@@ -16,6 +16,13 @@ shard with the all-gather of the estimates FUSED into the kernel that writes the
 buffer over NVLink), on-device error sums, NCCL all-reduce of the sums.  `value` times it with the inputs resident in
 HBM (CUDA events on the launch stream, one pair per step, L2 flushed between steps, max over ranks); `e2e` runs the same
 step from pinned HOST inputs to pinned host estimates (H2D / D2H inside the timed region).  Prints ONE JSON line (rank 0).
+
+--dump-outputs DIR (our arm): after the timed steps, rank 0 writes what the last timed step returned, so that two builds
+can be compared output for output on identical seeded inputs:
+  estimates.npy      float32 [n, 120, 14, 2]  all-gathered estimates (re, im) of n rows: all of them, or a fixed seeded
+                                              sample of DUMP_ROWS rows when the global batch is larger (64 MB at most)
+  estimate_rows.npy  float64 [n]              the global row index of each dumped estimate
+  error_sums.npy     float64 [2]              the reduced [sum |est - truth|^2, sum |truth|^2]
 """
 import argparse
 import hashlib
@@ -39,6 +46,7 @@ FORTI = dict(model_type="fortitran", patch_size=(3, 2), num_layers=6, model_dim=
              dropout=0.1, max_seq_len=512, pos_encoding_type="learnable")
 ADA = dict(FORTI, model_type="adafortitran", channel_adaptivity_hidden_sizes=[7, 42, 560], adaptive_token_length=6)
 ENCODER_SOURCES = ("tc_encoder.cu", "tc_ptx.cuh", "tc_layout.cuh", "tc_encoder.cuh", "tc_math.cuh")
+DUMP_ROWS = 4096                                          # 4096 x 120 x 14 x 2 float32 = 55 MB
 
 
 def parse():
@@ -57,6 +65,7 @@ def parse():
     ap.add_argument("--cpu-batch", type=int, default=64, help="reference arm: estimates per step (BASELINE configs[0])")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra_configs / collectives comparison legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/*.npy (our arm)")
     return ap.parse_args()
 
 
@@ -275,6 +284,19 @@ def timed_steps(ev, pilots, meta, truth, steps, flush, barrier, world, dev):
     return float(total_ms.item()), wall, gathered, sums
 
 
+def dump_outputs(out_dir, gathered, sums):
+    """Writes the step's outputs as described in the module docstring (--dump-outputs)."""
+    import numpy as np
+    import torch
+    n = gathered.shape[0]
+    rows = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(0).choice(n, DUMP_ROWS, replace=False))
+    est = torch.view_as_real(gathered[torch.from_numpy(rows).to(gathered.device)]).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "estimates.npy"), est.astype(np.float32, copy=False))
+    np.save(os.path.join(out_dir, "estimate_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "error_sums.npy"), sums.cpu().numpy().astype(np.float64, copy=False))
+
+
 def run_ours(args):
     import ctypes as C
     import torch
@@ -287,6 +309,8 @@ def run_ours(args):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if world != args.gpus:
         raise SystemExit(f"--gpus {args.gpus} but WORLD_SIZE={world}: launch with torchrun --nproc-per-node {args.gpus}")
+    if args.steps < 1:
+        raise SystemExit(f"--steps {args.steps}: at least one timed step is needed")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
@@ -341,6 +365,10 @@ def run_ours(args):
         value = GB * args.steps / (total_ms / 1e3)
         sums_host = sums.cpu()
         nmse_db = float(10.0 * torch.log10(sums_host[0] / sums_host[1]))
+        if args.dump_outputs:                   # before the e2e steps below overwrite the gather buffer and the sums
+            if rank == 0:
+                dump_outputs(args.dump_outputs, gathered, sums)
+            barrier()                           # no rank's e2e step stores into rank 0's gather buffer while it is read
         reference_out = gathered[rank * B:(rank + 1) * B].clone() if gathered is not None else None
 
         # ---- end to end: pinned host inputs -> (H2D, forward + fused gather, error sums, all-reduce) -> pinned host estimates
@@ -441,6 +469,8 @@ def run_ours(args):
 if __name__ == "__main__":
     a = parse()
     if a.impl == "reference":
+        if a.dump_outputs:
+            raise SystemExit("--dump-outputs applies to --impl ours")
         run_reference(a)
     else:
         run_ours(a)

@@ -1,6 +1,6 @@
 import json, os, sys, time
 import numpy as np, torch
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from adafortitran_b200 import AdaFortiTranEstimator, ModelConfig, SystemConfig
 from tests import util
 sysc = SystemConfig(ofdm=dict(num_scs=3276, num_symbols=14), pilot=dict(num_scs=1638, num_symbols=2))
