@@ -10,7 +10,7 @@ import ctypes as C
 import os
 import threading
 
-AFT_ABI_VERSION = 2
+AFT_ABI_VERSION = 3
 AFT_OK = 0
 AFT_ERR_INVALID, AFT_ERR_UNSUPPORTED, AFT_ERR_CUDA, AFT_ERR_WORKSPACE, AFT_ERR_STATE = -1, -2, -3, -4, -5
 AFT_FP32, AFT_BF16 = 0, 1
@@ -84,6 +84,11 @@ EXPORTS = {
     "aft_profile_enable": (C.c_int, [C.c_void_p, C.c_int]),
     "aft_profile_read": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     "aft_selftest": (C.c_int, [C.c_int, C.POINTER(C.c_double), C.c_void_p]),
+    "aft_param_count": (C.c_int64, [C.c_void_p]),
+    "aft_train_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_int64]),
+    "aft_forward_train": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                    C.c_float, C.c_uint64, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "aft_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
 }
 
 _LIB = None

@@ -2,6 +2,7 @@
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
+#include <cmath>
 #include <cstring>
 #include <new>
 #include <string>
@@ -9,6 +10,7 @@
 
 #include "aft_internal.cuh"
 #include "tc_encoder.cuh"
+#include "train.cuh"
 
 namespace aft {
 
@@ -779,3 +781,121 @@ int aft_selftest(int which, double* max_err, void* stream) {
 }
 
 }  // extern "C"
+
+// ---------------------------------------------------------------------------------------------
+// training path (train_fwd.cu / train_bwd.cu)
+// ---------------------------------------------------------------------------------------------
+namespace {
+
+TrainModel train_model(const AftHandle* h) {
+  return TrainModel{&h->front, &h->head, h->layers.data(), h->cfg.num_layers, h->cfg.activation, h->cfg.adaptive,
+                    h->cfg.adapt_h1, h->cfg.adapt_h2, h->cfg.max_seq_len};
+}
+
+int train_unsupported(const char* fn) {
+  set_error("%s: training covers only the reference default geometry (grid 120x14, pilots 12x2, patch 3x2)", fn);
+  return AFT_ERR_UNSUPPORTED;
+}
+
+// common checks of aft_forward_train / aft_backward; fills *ws when the workspace is usable
+int train_check_ws(const AftHandle* h, const char* fn, int64_t batch, void* workspace, size_t workspace_bytes, TrainWs* ws) {
+  const size_t need = train_layout(nullptr, batch, h->cfg.num_layers).bytes;
+  if (!workspace || workspace_bytes < need) {
+    set_error("%s: workspace too small (%zu < %zu bytes)", fn, workspace_bytes, need);
+    return AFT_ERR_WORKSPACE;
+  }
+  if ((reinterpret_cast<uintptr_t>(workspace) & 255) != 0) {
+    set_error("%s: workspace must be 256-byte aligned", fn);
+    return AFT_ERR_WORKSPACE;
+  }
+  *ws = train_layout(workspace, batch, h->cfg.num_layers);
+  return AFT_OK;
+}
+
+DropCfg drop_cfg(float p, uint64_t seed) {
+  DropCfg d;
+  d.thresh = (uint32_t)std::floor((double)p * 4294967296.0);
+  d.scale = 1.0f / (1.0f - p);
+  d.seed_lo = (uint32_t)(seed & 0xffffffffu);
+  d.seed_hi = (uint32_t)(seed >> 32);
+  return d;
+}
+
+}  // namespace
+
+extern "C" {
+
+int64_t aft_param_count(const AftHandle* h) {
+  if (!h) { set_error("aft_param_count: NULL handle"); return 0; }
+  if (h->generic) { train_unsupported("aft_param_count"); return 0; }
+  return (int64_t)grad_layout(train_model(h)).total;
+}
+
+size_t aft_train_workspace_bytes(const AftHandle* h, int64_t batch) {
+  if (!h || batch < 0) { set_error("aft_train_workspace_bytes: bad argument"); return 0; }
+  if (h->generic) { train_unsupported("aft_train_workspace_bytes"); return 0; }
+  return train_layout(nullptr, batch, h->cfg.num_layers).bytes;
+}
+
+int aft_forward_train(AftHandle* h, const void* pilots, const float* snr, const float* delay_spread, const float* doppler,
+                      void* out, int64_t batch, float dropout, uint64_t seed, void* workspace, size_t workspace_bytes,
+                      void* stream) {
+  if (!h) { set_error("aft_forward_train: NULL handle"); return AFT_ERR_INVALID; }
+  if (h->generic) return train_unsupported("aft_forward_train");
+  if (!(dropout >= 0.f && dropout < 1.f)) { set_error("aft_forward_train: dropout %g outside [0, 1)", (double)dropout); return AFT_ERR_INVALID; }
+  if (batch < 0) { set_error("aft_forward_train: negative batch"); return AFT_ERR_INVALID; }
+  if (!h->loaded) { set_error("aft_forward_train: weights not loaded (call aft_load_weights first)"); return AFT_ERR_STATE; }
+  if (batch == 0) return AFT_OK;
+  if (!pilots || !out) { set_error("aft_forward_train: NULL pilots / out"); return AFT_ERR_INVALID; }
+  if (h->cfg.adaptive && (!snr || !delay_spread || !doppler)) {
+    set_error("aft_forward_train: meta_data is required when channel adaptation is enabled");
+    return AFT_ERR_INVALID;
+  }
+  TrainWs ws;
+  const int rc = train_check_ws(h, "aft_forward_train", batch, workspace, workspace_bytes, &ws);
+  if (rc != AFT_OK) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const DropCfg drop = drop_cfg(dropout, seed);
+  // the header record tells aft_backward which forward filled the workspace (written on the device by the first kernel)
+  const TrainHeader hdr{kTrainMagic, batch, h->cfg.num_layers, h->cfg.adaptive, dropout, drop.thresh, seed};
+  if (!train_forward(train_model(h), hdr, static_cast<const float2*>(pilots), snr, delay_spread, doppler, static_cast<float2*>(out),
+                     batch, drop, ws, st))
+    return AFT_ERR_CUDA;
+  return AFT_OK;
+}
+
+int aft_backward(AftHandle* h, const void* grad_out, int64_t batch, void* workspace, size_t workspace_bytes, float* grads,
+                 void* stream) {
+  if (!h) { set_error("aft_backward: NULL handle"); return AFT_ERR_INVALID; }
+  if (h->generic) return train_unsupported("aft_backward");
+  if (batch < 0) { set_error("aft_backward: negative batch"); return AFT_ERR_INVALID; }
+  if (!h->loaded) { set_error("aft_backward: weights not loaded (call aft_load_weights first)"); return AFT_ERR_STATE; }
+  if (batch == 0) return AFT_OK;
+  if (!grad_out || !grads) { set_error("aft_backward: NULL grad_out / grads"); return AFT_ERR_INVALID; }
+  if (!workspace || workspace_bytes < sizeof(TrainHeader) || (reinterpret_cast<uintptr_t>(workspace) & 255) != 0) {
+    set_error("aft_backward: workspace NULL, too small or not 256-byte aligned");
+    return AFT_ERR_WORKSPACE;
+  }
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  // the header record of the forward: a 40-byte read-back, so this call synchronises with `stream`
+  TrainHeader hdr{};
+  AFT_CUDA(cudaMemcpyAsync(&hdr, workspace, sizeof(hdr), cudaMemcpyDeviceToHost, st));
+  AFT_CUDA(cudaStreamSynchronize(st));
+  if (hdr.magic != kTrainMagic || hdr.layers != h->cfg.num_layers || hdr.adaptive != h->cfg.adaptive) {
+    set_error("aft_backward: the workspace was not filled by aft_forward_train of this estimator");
+    return AFT_ERR_INVALID;
+  }
+  if (hdr.batch != batch) {
+    set_error("aft_backward: batch %lld differs from the forward's %lld", (long long)batch, (long long)hdr.batch);
+    return AFT_ERR_INVALID;
+  }
+  TrainWs ws;
+  const int rc = train_check_ws(h, "aft_backward", batch, workspace, workspace_bytes, &ws);
+  if (rc != AFT_OK) return rc;
+  if (!train_backward(train_model(h), static_cast<const float2*>(grad_out), batch, drop_cfg(hdr.dropout, hdr.seed), ws, grads, st))
+    return AFT_ERR_CUDA;
+  return AFT_OK;
+}
+
+}  // extern "C"
+

@@ -4,8 +4,10 @@
 //   kEpiBias       : QKV projection
 //   kEpiBiasAct    : FFN linear1 + GELU(erf) / ReLU
 //   kEpiBiasResLn  : out_proj / linear2 + residual + LayerNorm (N == 128 == one tile, statistics tile-local)
+// and the two epilogues of the training forward (train.cuh), which add dropout and keep the pre-LN sum / the
+// pre-activation for the backward; with p = 0 they compute exactly what kEpiBiasResLn / kEpiBiasAct compute.
 // Plain FMA accumulation (no TF32): the fp32 parity gate is 1e-4 normwise.
-#include "aft_internal.cuh"
+#include "train.cuh"
 
 namespace aft {
 
@@ -17,7 +19,8 @@ template <int EPI>
 __global__ void __launch_bounds__(256)
 gemm_f32_kernel(const float* __restrict__ A, const float* __restrict__ W, const float* __restrict__ bias,
                 float* C, int64_t M, int N, int K, int act, const float* residual,
-                const float* __restrict__ gamma, const float* __restrict__ beta) {
+                const float* __restrict__ gamma, const float* __restrict__ beta, TrainEpi te) {
+  constexpr bool kResLn = EPI == kEpiBiasResLn || EPI == kEpiTrainResLn;
   __shared__ __align__(16) float As[BK][PITCH];
   __shared__ __align__(16) float Bs[BK][PITCH];
   const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
@@ -64,7 +67,7 @@ gemm_f32_kernel(const float* __restrict__ A, const float* __restrict__ W, const 
   const float4 biasB = *reinterpret_cast<const float4*>(bias + cB);
   const float bv[8] = {biasA.x, biasA.y, biasA.z, biasA.w, biasB.x, biasB.y, biasB.z, biasB.w};
   float gv[8], be[8];
-  if (EPI == kEpiBiasResLn) {
+  if (kResLn) {
     const float4 gA = *reinterpret_cast<const float4*>(gamma + cA), gB = *reinterpret_cast<const float4*>(gamma + cB);
     const float4 eA = *reinterpret_cast<const float4*>(beta + cA), eB = *reinterpret_cast<const float4*>(beta + cB);
     gv[0] = gA.x; gv[1] = gA.y; gv[2] = gA.z; gv[3] = gA.w; gv[4] = gB.x; gv[5] = gB.y; gv[6] = gB.z; gv[7] = gB.w;
@@ -77,16 +80,32 @@ gemm_f32_kernel(const float* __restrict__ A, const float* __restrict__ W, const 
     float v[8];
 #pragma unroll
     for (int j = 0; j < 8; ++j) v[j] = acc[i][j] + bv[j];
-    if (EPI == kEpiBiasAct) {
+    if (EPI == kEpiTrainAct && live) {
+      *reinterpret_cast<float4*>(te.aux + m * N + cA) = make_float4(v[0], v[1], v[2], v[3]);
+      *reinterpret_cast<float4*>(te.aux + m * N + cB) = make_float4(v[4], v[5], v[6], v[7]);
+    }
+    if (EPI == kEpiBiasAct || EPI == kEpiTrainAct) {
 #pragma unroll
       for (int j = 0; j < 8; ++j) v[j] = act == AFT_ACT_GELU ? gelu_erf(v[j]) : fmaxf(v[j], 0.f);
     }
-    if (EPI == kEpiBiasResLn) {
+    if ((EPI == kEpiTrainAct || EPI == kEpiTrainResLn) && te.drop.thresh != 0u) {
+      // element index row * N + col within the sequence; cA and cB are multiples of 4: one Philox call each
+      const uint32_t seq = (uint32_t)(m / kS), row = (uint32_t)(m - (int64_t)seq * kS);
+      const float4 ka = te.drop.mult4((row * N + cA) >> 2, seq, te.layer_site);
+      const float4 kb = te.drop.mult4((row * N + cB) >> 2, seq, te.layer_site);
+      v[0] *= ka.x; v[1] *= ka.y; v[2] *= ka.z; v[3] *= ka.w;
+      v[4] *= kb.x; v[5] *= kb.y; v[6] *= kb.z; v[7] *= kb.w;
+    }
+    if (kResLn) {
       if (live) {
         const float4 rA = *reinterpret_cast<const float4*>(residual + m * N + cA);
         const float4 rB = *reinterpret_cast<const float4*>(residual + m * N + cB);
         v[0] += rA.x; v[1] += rA.y; v[2] += rA.z; v[3] += rA.w;
         v[4] += rB.x; v[5] += rB.y; v[6] += rB.z; v[7] += rB.w;
+        if (EPI == kEpiTrainResLn) {
+          *reinterpret_cast<float4*>(te.aux + m * N + cA) = make_float4(v[0], v[1], v[2], v[3]);
+          *reinterpret_cast<float4*>(te.aux + m * N + cB) = make_float4(v[4], v[5], v[6], v[7]);
+        }
       }
       float s = 0.f;
 #pragma unroll
@@ -180,17 +199,35 @@ bool launch_gemm_f32(int epi, const float* A, const float* W, const float* bias,
     return false;
   }
   const dim3 grid((unsigned)((M + BM - 1) / BM), (unsigned)(N / BN));
+  const TrainEpi none{};
   switch (epi) {
     case kEpiBias:
-      gemm_f32_kernel<kEpiBias><<<grid, 256, 0, st>>>(A, W, bias, C, M, N, K, act, residual, gamma, beta);
+      gemm_f32_kernel<kEpiBias><<<grid, 256, 0, st>>>(A, W, bias, C, M, N, K, act, residual, gamma, beta, none);
       break;
     case kEpiBiasAct:
-      gemm_f32_kernel<kEpiBiasAct><<<grid, 256, 0, st>>>(A, W, bias, C, M, N, K, act, residual, gamma, beta);
+      gemm_f32_kernel<kEpiBiasAct><<<grid, 256, 0, st>>>(A, W, bias, C, M, N, K, act, residual, gamma, beta, none);
       break;
     default:
-      gemm_f32_kernel<kEpiBiasResLn><<<grid, 256, 0, st>>>(A, W, bias, C, M, N, K, act, residual, gamma, beta);
+      gemm_f32_kernel<kEpiBiasResLn><<<grid, 256, 0, st>>>(A, W, bias, C, M, N, K, act, residual, gamma, beta, none);
       break;
   }
+  count_launch();
+  return check_launch("gemm_f32_kernel");
+}
+
+bool launch_gemm_f32_train(int epi, const float* A, const float* W, const float* bias, float* C, int64_t M, int N, int K,
+                           int act, const float* residual, const float* gamma, const float* beta, const TrainEpi& te,
+                           cudaStream_t st) {
+  if (M <= 0) return true;
+  if (N % BN != 0 || K % BK != 0 || (epi == kEpiTrainResLn && N != BN) || (epi != kEpiTrainResLn && epi != kEpiTrainAct)) {
+    set_error("gemm_f32_train: unsupported shape N=%d K=%d epi=%d", N, K, epi);
+    return false;
+  }
+  const dim3 grid((unsigned)((M + BM - 1) / BM), (unsigned)(N / BN));
+  if (epi == kEpiTrainResLn)
+    gemm_f32_kernel<kEpiTrainResLn><<<grid, 256, 0, st>>>(A, W, bias, C, M, N, K, act, residual, gamma, beta, te);
+  else
+    gemm_f32_kernel<kEpiTrainAct><<<grid, 256, 0, st>>>(A, W, bias, C, M, N, K, act, residual, gamma, beta, te);
   count_launch();
   return check_launch("gemm_f32_kernel");
 }

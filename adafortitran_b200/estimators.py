@@ -148,7 +148,15 @@ class BaseFortiTranEstimator(nn.Module):
 
     ``precision``: ``"fp32"`` (CUDA-core path, <= 1e-4 normwise vs the reference) or ``"bf16"`` (tcgen05
     path).  Default from ``$AFT_PRECISION``, else ``"fp32"``.
+
+    ``trainable`` (default ``False``): with ``True``, a ``forward`` with grad enabled is differentiable with respect to
+    every parameter (fp32 CUDA-core training path, reference default geometry): it applies the reference's dropout
+    (``model_config.dropout``) in ``train()`` mode and none in ``eval()`` mode, and ``loss.backward()`` fills ``.grad``
+    through ``aft_backward``.  Dropout masks are drawn from torch's default generator, so ``torch.manual_seed`` makes
+    runs reproducible.
     """
+
+    trainable = False
 
     def __init__(self, system_config: SystemConfig, model_config: ModelConfig,
                  use_channel_adaptation: bool = False) -> None:
@@ -371,9 +379,12 @@ class BaseFortiTranEstimator(nn.Module):
             raise ValueError("meta_data is required when channel adaptation is enabled")
         if not self.use_channel_adaptation and meta_data is not None:
             self.logger.warning("meta_data provided but channel adaptation is disabled - ignoring meta_data")
-        if self.training and torch.is_grad_enabled():
-            raise RuntimeError("this implementation is inference-only: call model.eval() and/or run under "
-                               "torch.no_grad() (the reference training loop is out of scope)")
+        if where == "cpu" and self.trainable and torch.is_grad_enabled():
+            raise RuntimeError("forward_host is inference-only and not differentiable: with model.trainable = True and "
+                               "grad enabled, call forward() on device tensors, or run forward_host under torch.no_grad()")
+        if self.training and torch.is_grad_enabled() and not (self.trainable and where == "cuda"):
+            raise RuntimeError("this implementation is inference-only unless model.trainable = True: call model.eval() "
+                               "and/or run under torch.no_grad(), or set model.trainable = True to train on the GPU")
         if not torch.is_tensor(pilot_symbols) or not torch.is_complex(pilot_symbols):
             raise TypeError(f"pilot_symbols must be a complex tensor, got {getattr(pilot_symbols, 'dtype', type(pilot_symbols))}")
         if pilot_symbols.dim() != 3 or tuple(pilot_symbols.shape[1:]) != self.pilot_size:
@@ -419,6 +430,8 @@ class BaseFortiTranEstimator(nn.Module):
         local gather buffer."""
         precision = self._precision_code()
         batch, cond_in = self._check_call(pilot_symbols, meta_data, "cuda")
+        if self.trainable and torch.is_grad_enabled():
+            return self._forward_differentiable(pilot_symbols, cond_in, batch, precision, gather)
         self._ensure_handle()
         with torch.cuda.device(self.device):
             pilots = pilot_symbols.to(device=self.device, dtype=torch.complex64).contiguous()
@@ -450,6 +463,27 @@ class BaseFortiTranEstimator(nn.Module):
                     self._handle, vp(pilots), vp(cond[0]), vp(cond[1]), vp(cond[2]), vp(stage), batch, precision,
                     C.c_void_p(ws_ptr), ws.numel() - (ws_ptr - ws.data_ptr()), C.c_void_p(stream), C.byref(plan)))
         return out
+
+    def _forward_differentiable(self, pilot_symbols, cond_in, batch, precision, gather) -> torch.Tensor:
+        if precision != _capi.AFT_FP32:
+            raise ValueError("training (trainable = True with grad enabled) runs on the fp32 CUDA-core path only; "
+                             "set model.precision = 'fp32' or run under torch.no_grad()")
+        if gather is not None:
+            raise ValueError("gather= is an inference path: it cannot be combined with a differentiable call")
+        inputs = [pilot_symbols] + list(cond_in or [])
+        if any(torch.is_tensor(t) and t.requires_grad for t in inputs):
+            raise ValueError("gradients with respect to the pilots or the metadata are not computed: pass inputs that "
+                             "do not require grad")
+        self._ensure_handle()
+        with torch.cuda.device(self.device):
+            pilots = pilot_symbols.to(device=self.device, dtype=torch.complex64).contiguous()
+            cond = [None, None, None]
+            if cond_in is not None:
+                cond = [t.to(device=self.device, dtype=torch.float32).reshape(-1).contiguous() for t in cond_in]
+            p = float(self.model_config.dropout) if self.training else 0.0
+            seed = int(torch.randint(0, 2 ** 62, (), dtype=torch.int64).item())
+            named, _ = self._weight_tensors()
+            return _TrainForward.apply(self, pilots, cond, batch, p, seed, *[t for _, t in named])
 
     def forward_host(self, pilot_symbols: torch.Tensor, meta_data: Optional[Tuple] = None,
                      out: Optional[torch.Tensor] = None, gather=None) -> torch.Tensor:
@@ -485,6 +519,58 @@ class BaseFortiTranEstimator(nn.Module):
         out = super()._load_from_state_dict(*args, **kwargs)
         self._packed_key = None     # load_state_dict: always repack (copy_ into .data would otherwise go unnoticed)
         return out
+
+
+class _TrainForward(torch.autograd.Function):
+    """``aft_forward_train`` / ``aft_backward`` behind autograd.  The parameters are inputs of the Function (in the order
+    of ``_weight_tensors``), so ``AccumulateGrad``, ``requires_grad=False``, hooks and version checks work as for any
+    torch op; their gradients are views of the flat buffer ``aft_backward`` fills."""
+
+    @staticmethod
+    def forward(ctx, model, pilots, cond, batch, p, seed, *params):
+        model._sync_weights()
+        out = torch.empty((batch, *model.ofdm_size), dtype=torch.complex64, device=model.device)
+        ws = None
+        if batch > 0:
+            lib = _capi.lib()
+            need = lib.aft_train_workspace_bytes(model._handle, batch)
+            if need == 0:
+                _capi.check(_capi.AFT_ERR_UNSUPPORTED if model._handle else _capi.AFT_ERR_INVALID)
+            ws = torch.empty(need + 256, dtype=torch.uint8, device=model.device)
+            ws_ptr = (ws.data_ptr() + 255) // 256 * 256
+            vp = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+            stream = torch.cuda.current_stream(model.device).cuda_stream
+            _capi.check(lib.aft_forward_train(model._handle, vp(pilots), vp(cond[0]), vp(cond[1]), vp(cond[2]), vp(out),
+                                              batch, p, seed, C.c_void_p(ws_ptr), need, C.c_void_p(stream)))
+        ctx.model, ctx.batch, ctx.ws = model, batch, ws
+        ctx.save_for_backward(*params)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        params = ctx.saved_tensors    # raises if a parameter was modified in place since the forward
+        model, batch, ws = ctx.model, ctx.batch, ctx.ws
+        if ws is None and batch > 0:
+            raise RuntimeError("backward through the same training forward a second time: the saved activations were "
+                               "released after the first backward (retain_graph is not supported)")
+        ctx.ws = None
+        lib = _capi.lib()
+        n = lib.aft_param_count(model._handle)
+        flat = torch.zeros(n, dtype=torch.float32, device=model.device)
+        if batch > 0:
+            g = torch.view_as_real(grad_out.to(torch.complex64).resolve_conj()).contiguous()
+            ws_ptr = (ws.data_ptr() + 255) // 256 * 256
+            need = lib.aft_train_workspace_bytes(model._handle, batch)
+            with torch.cuda.device(model.device):
+                stream = torch.cuda.current_stream(model.device).cuda_stream
+                _capi.check(lib.aft_backward(model._handle, C.c_void_p(g.data_ptr()), batch, C.c_void_p(ws_ptr), need,
+                                             C.c_void_p(flat.data_ptr()), C.c_void_p(stream)))
+        grads, off = [], 0
+        for i, t in enumerate(params):
+            k = t.numel()
+            grads.append(flat[off:off + k].view(t.shape).to(t.dtype) if ctx.needs_input_grad[6 + i] else None)
+            off += k
+        return (None, None, None, None, None, None, *grads)
 
 
 class FortiTranEstimator(BaseFortiTranEstimator):

@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define AFT_ABI_VERSION 2
+#define AFT_ABI_VERSION 3
 
 #if defined(__GNUC__)
 #define AFT_API __attribute__((visibility("default")))
@@ -195,6 +195,40 @@ AFT_API int64_t aft_launch_count(void);
  * launches per stage, and resets the accumulators.  fp32 path: "encoder" covers its GEMM + attention kernels. */
 AFT_API int aft_profile_enable(AftHandle* h, int enable);
 AFT_API int aft_profile_read(AftHandle* h, double* ms, int64_t* launches);
+
+/* ---- Training (AFT_FP32 on CUDA cores, reference default geometry only) ----------------------------------------
+ * A handle on any other geometry returns AFT_ERR_UNSUPPORTED from the four calls below.
+ *
+ * Flat gradient layout: every parameter in torch layout without padding, in this order:
+ *   pilot_upsampler w, b;  initial_enhancer w0 b0 w1 b1 w2 b2 w3 b3;  final_refiner w0 b0 .. w3 b3;
+ *   (adaptive only) snr_encoder w0 b0 w1 b1 w2 b2, ds_encoder ..., dop_encoder ...;
+ *   linear_1 w, b;  positional table [max_seq_len, model_dim] (rows >= 280 are 0);  linear_2 w, b;
+ *   per encoder layer: in_proj w b, out_proj w b, linear1 w b, linear2 w b, norm1 w b, norm2 w b.
+ *
+ * Dropout: nn.TransformerEncoderLayer's four sites (post-norm): 0 the attention probabilities, element index
+ * (head*S + q)*S + k; 1 the out_proj output before the residual add, row*128 + col; 2 the FFN activation,
+ * row*256 + col; 3 the linear2 output before the residual add, row*128 + col (row = token of the sequence).
+ * Element i of sequence seq (= sample*2 + {0 re, 1 im}) in layer l at site s takes output word i & 3 of
+ * Philox4x32-10 with key (seed & 0xffffffff, seed >> 32) and counter (i >> 2, seq, (l << 8) | s, 0), and is kept
+ * iff that word >= floor(p * 2^32) (p as float, widened to double); kept values are scaled by 1 / (1 - p). */
+
+/* Floats in the flat gradient buffer of aft_backward (0 on error). */
+AFT_API int64_t aft_param_count(const AftHandle* h);
+/* Bytes of the training workspace for `batch` samples: saved activations + backward scratch (0 on error). */
+AFT_API size_t aft_train_workspace_bytes(const AftHandle* h, int64_t batch);
+/* Training forward, AFT_FP32 only: as aft_forward, plus dropout with probability `dropout` (0 <= p < 1) at the four
+ * sites of nn.TransformerEncoderLayer, masks drawn from `seed` (see "Dropout" above); saves what aft_backward needs in
+ * `workspace` (256-byte aligned).  Asynchronous on `stream`, no allocation, no host synchronisation.  With p = 0 the
+ * output is bit-identical to aft_forward at AFT_FP32. */
+AFT_API int aft_forward_train(AftHandle* h, const void* pilots, const float* snr, const float* delay_spread,
+                              const float* doppler, void* out, int64_t batch, float dropout, uint64_t seed,
+                              void* workspace, size_t workspace_bytes, void* stream);
+/* Gradients of all parameters for grad_out = dL/d(out) (complex64 [batch, num_scs, num_symbols]: re = dL/dRe, im = dL/dIm).
+ * Overwrites grads[aft_param_count(h)] (fp32, device).  Consumes the workspace of the aft_forward_train call it follows;
+ * reads that call's header record back first (so it synchronises with `stream`) and returns AFT_ERR_INVALID when
+ * `batch` differs from it.  Deterministic: the same inputs and seed give bit-identical gradients. */
+AFT_API int aft_backward(AftHandle* h, const void* grad_out, int64_t batch, void* workspace, size_t workspace_bytes,
+                         float* grads, void* stream);
 
 /* Device-side self tests of the tcgen05 building blocks against SIMT code (returns max abs error in
  * *max_err; used by tests/ to localise failures).  which: 0 = UMMA GEMM tile, 1 = attention tile. */
