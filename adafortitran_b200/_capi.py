@@ -88,6 +88,9 @@ EXPORTS = {
     "aft_train_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_int64]),
     "aft_forward_train": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                     C.c_float, C.c_uint64, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "aft_forward_train_offset": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_int64, C.c_int64, C.c_float, C.c_uint64, C.c_void_p, C.c_size_t,
+                                           C.c_void_p]),
     "aft_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
 }
 

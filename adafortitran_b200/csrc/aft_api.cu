@@ -812,12 +812,13 @@ int train_check_ws(const AftHandle* h, const char* fn, int64_t batch, void* work
   return AFT_OK;
 }
 
-DropCfg drop_cfg(float p, uint64_t seed) {
+DropCfg drop_cfg(float p, uint64_t seed, int64_t sample0) {
   DropCfg d;
   d.thresh = (uint32_t)std::floor((double)p * 4294967296.0);
   d.scale = 1.0f / (1.0f - p);
   d.seed_lo = (uint32_t)(seed & 0xffffffffu);
   d.seed_hi = (uint32_t)(seed >> 32);
+  d.seq0 = (uint32_t)(2 * sample0);   // < 2^32: checked by aft_forward_train_offset
   return d;
 }
 
@@ -837,13 +838,19 @@ size_t aft_train_workspace_bytes(const AftHandle* h, int64_t batch) {
   return train_layout(nullptr, batch, h->cfg.num_layers).bytes;
 }
 
-int aft_forward_train(AftHandle* h, const void* pilots, const float* snr, const float* delay_spread, const float* doppler,
-                      void* out, int64_t batch, float dropout, uint64_t seed, void* workspace, size_t workspace_bytes,
-                      void* stream) {
+int aft_forward_train_offset(AftHandle* h, const void* pilots, const float* snr, const float* delay_spread,
+                             const float* doppler, void* out, int64_t batch, int64_t sample0, float dropout, uint64_t seed,
+                             void* workspace, size_t workspace_bytes, void* stream) {
   if (!h) { set_error("aft_forward_train: NULL handle"); return AFT_ERR_INVALID; }
   if (h->generic) return train_unsupported("aft_forward_train");
   if (!(dropout >= 0.f && dropout < 1.f)) { set_error("aft_forward_train: dropout %g outside [0, 1)", (double)dropout); return AFT_ERR_INVALID; }
   if (batch < 0) { set_error("aft_forward_train: negative batch"); return AFT_ERR_INVALID; }
+  // the global sequence index 2 * (sample0 + b) + part is the 32-bit second word of the Philox counter
+  if (sample0 < 0 || sample0 > (int64_t{1} << 31) - batch) {
+    set_error("aft_forward_train: samples [%lld, %lld) outside [0, 2^31)", (long long)sample0,
+              (long long)sample0 + (long long)batch);
+    return AFT_ERR_INVALID;
+  }
   if (!h->loaded) { set_error("aft_forward_train: weights not loaded (call aft_load_weights first)"); return AFT_ERR_STATE; }
   if (batch == 0) return AFT_OK;
   if (!pilots || !out) { set_error("aft_forward_train: NULL pilots / out"); return AFT_ERR_INVALID; }
@@ -855,13 +862,20 @@ int aft_forward_train(AftHandle* h, const void* pilots, const float* snr, const 
   const int rc = train_check_ws(h, "aft_forward_train", batch, workspace, workspace_bytes, &ws);
   if (rc != AFT_OK) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const DropCfg drop = drop_cfg(dropout, seed);
+  const DropCfg drop = drop_cfg(dropout, seed, sample0);
   // the header record tells aft_backward which forward filled the workspace (written on the device by the first kernel)
-  const TrainHeader hdr{kTrainMagic, batch, h->cfg.num_layers, h->cfg.adaptive, dropout, drop.thresh, seed};
+  const TrainHeader hdr{kTrainMagic, batch, h->cfg.num_layers, h->cfg.adaptive, dropout, drop.thresh, seed, sample0};
   if (!train_forward(train_model(h), hdr, static_cast<const float2*>(pilots), snr, delay_spread, doppler, static_cast<float2*>(out),
                      batch, drop, ws, st))
     return AFT_ERR_CUDA;
   return AFT_OK;
+}
+
+int aft_forward_train(AftHandle* h, const void* pilots, const float* snr, const float* delay_spread, const float* doppler,
+                      void* out, int64_t batch, float dropout, uint64_t seed, void* workspace, size_t workspace_bytes,
+                      void* stream) {
+  return aft_forward_train_offset(h, pilots, snr, delay_spread, doppler, out, batch, 0, dropout, seed, workspace,
+                                  workspace_bytes, stream);
 }
 
 int aft_backward(AftHandle* h, const void* grad_out, int64_t batch, void* workspace, size_t workspace_bytes, float* grads,
@@ -877,7 +891,7 @@ int aft_backward(AftHandle* h, const void* grad_out, int64_t batch, void* worksp
     return AFT_ERR_WORKSPACE;
   }
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  // the header record of the forward: a 40-byte read-back, so this call synchronises with `stream`
+  // the header record of the forward: a 48-byte read-back, so this call synchronises with `stream`
   TrainHeader hdr{};
   AFT_CUDA(cudaMemcpyAsync(&hdr, workspace, sizeof(hdr), cudaMemcpyDeviceToHost, st));
   AFT_CUDA(cudaStreamSynchronize(st));
@@ -892,7 +906,8 @@ int aft_backward(AftHandle* h, const void* grad_out, int64_t batch, void* worksp
   TrainWs ws;
   const int rc = train_check_ws(h, "aft_backward", batch, workspace, workspace_bytes, &ws);
   if (rc != AFT_OK) return rc;
-  if (!train_backward(train_model(h), static_cast<const float2*>(grad_out), batch, drop_cfg(hdr.dropout, hdr.seed), ws, grads, st))
+  const DropCfg drop = drop_cfg(hdr.dropout, hdr.seed, hdr.sample0);
+  if (!train_backward(train_model(h), static_cast<const float2*>(grad_out), batch, drop, ws, grads, st))
     return AFT_ERR_CUDA;
   return AFT_OK;
 }

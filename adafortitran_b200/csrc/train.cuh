@@ -10,8 +10,9 @@ namespace aft {
 
 // ---------------------------------------------------------------------------------------------
 // Dropout rule (include/aft.h, "Dropout"): Philox4x32-10, key (seed_lo, seed_hi), counter
-// (i >> 2, seq, (layer << 8) | site, 0); element i uses output word i & 3 and is kept iff that word >= thresh,
-// thresh = floor(p * 2^32).  Kept values are scaled by 1 / (1 - p).
+// (i >> 2, seq0 + seq, (layer << 8) | site, 0) with seq the call-local sequence and seq0 = 2 * sample0 the first global
+// sequence of the call; element i uses output word i & 3 and is kept iff that word >= thresh, thresh = floor(p * 2^32).
+// Kept values are scaled by 1 / (1 - p).
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1) {
 #pragma unroll
@@ -29,8 +30,9 @@ struct DropCfg {
   uint32_t thresh;      // floor(p * 2^32); 0 = no dropout
   float scale;          // 1 / (1 - p)
   uint32_t seed_lo, seed_hi;
+  uint32_t seq0;        // 2 * sample0: global sequence index of the call's first sequence
   __device__ __forceinline__ uint4 words(uint32_t i4, uint32_t seq, uint32_t layer_site) const {
-    return philox4x32_10(make_uint4(i4, seq, layer_site, 0u), seed_lo, seed_hi);
+    return philox4x32_10(make_uint4(i4, seq0 + seq, layer_site, 0u), seed_lo, seed_hi);
   }
   // multipliers (0 or scale) of the four elements 4*i4 .. 4*i4+3
   __device__ __forceinline__ float4 mult4(uint32_t i4, uint32_t seq, uint32_t layer_site) const {
@@ -69,6 +71,7 @@ struct TrainHeader {
   float dropout;
   uint32_t thresh;
   uint64_t seed;
+  int64_t sample0;      // global index of the forward's first sample (aft_forward_train_offset)
 };
 constexpr uint64_t kTrainMagic = 0x31574b5254544641ull;   // "AFTTRKW1"
 constexpr int kMaxChunks = 128;                          // partial tiles of the deterministic weight-gradient sums

@@ -1,4 +1,5 @@
-"""Multi-GPU plumbing of the evaluation path: independent replicas, batch-sharded.
+"""Multi-GPU plumbing: batch-sharded evaluation (:class:`ShardedEvaluator`) and data-parallel training
+(:class:`ShardedTrainer`) over the GPUs of one node.
 
 The forward pass has no cross-sample arithmetic (reference ``src/models/fortitran.py:184-233``), so the only
 collectives of the path are the ones that follow it in the evaluator (SURVEY.md 8e): an all-gather of the
@@ -212,3 +213,85 @@ class ShardedEvaluator:
         if self.peer is not None:
             self.peer.close()
             self.peer = None
+
+
+class ShardedTrainer:
+    """Data-parallel training step over the ranks of ``group`` (one process and one GPU each): the training counterpart
+    of :class:`ShardedEvaluator`.
+
+    Each rank holds a replica of ``model`` (``trainable = True``, ``precision = "fp32"``) and the shard
+    ``shard_range(global_batch, rank, world)`` of every global batch.  :meth:`step` makes the ranks compute, together,
+    exactly what one call over the global batch computes:
+
+    * dropout: one seed per step, drawn on rank 0 from its default generator (as a single-GPU call draws it) and
+      broadcast; every rank forwards with ``sample_offset`` = its first global sample, so each sample gets the masks it
+      gets in a single call over the global batch, whatever ``torch.manual_seed`` each rank ran;
+    * loss: the reference's ``MSELoss`` over ``cat(re, im)`` of the global batch.  Each rank normalises its sum of
+      squared errors by the global batch, so unequal shards weigh every sample the same;
+    * gradients: one SUM all-reduce of one flat buffer holding every parameter gradient (and the loss).
+
+    Construction is collective: it broadcasts the parameters and buffers of rank 0, so the replicas start identical.
+    The caller keeps the optimizer: identical gradients on identical parameters give identical updates on every rank.
+    """
+
+    def __init__(self, model, group=None):
+        if not getattr(model, "trainable", False):
+            raise ValueError("ShardedTrainer needs a model with trainable = True")
+        if getattr(model, "precision", None) != "fp32":
+            raise ValueError(f"ShardedTrainer trains on the fp32 path only, the model has precision "
+                             f"{getattr(model, 'precision', None)!r}")
+        self.model, self.group = model, group
+        self._dist = dist.is_available() and dist.is_initialized()
+        self.world = dist.get_world_size(group) if self._dist else 1
+        self.rank = dist.get_rank(group) if self._dist else 0
+        self._src = dist.get_global_rank(group, 0) if self._dist and group is not None else 0
+        # NCCL moves device tensors, gloo host tensors
+        self._comm_device = model.device if self._dist and dist.get_backend(group) == "nccl" else torch.device("cpu")
+        self.params = [p for p in model.parameters() if p.requires_grad]
+        if self.world > 1:
+            with torch.no_grad():
+                for t in list(model.parameters()) + list(model.buffers()):
+                    buf = t.detach().to(self._comm_device, copy=True)
+                    dist.broadcast(buf, src=self._src, group=group)
+                    t.copy_(buf)     # in place through autograd's view: bumps the version, so packed copies refresh
+
+    def _seed(self) -> int:
+        seed = torch.randint(0, 2 ** 62, (), dtype=torch.int64) if self.rank == 0 else torch.zeros((), dtype=torch.int64)
+        if self.world > 1:
+            seed = seed.to(self._comm_device)
+            dist.broadcast(seed, src=self._src, group=self.group)
+        return int(seed.item())
+
+    def step(self, pilots_local, meta_local, truth_local: torch.Tensor, global_batch: int) -> torch.Tensor:
+        """Forward and backward of this rank's shard of a ``global_batch``-sample batch, then the gradient all-reduce.
+
+        ``pilots_local`` / ``meta_local`` / ``truth_local`` (complex ``[b, scs, symbols]``) hold samples ``[lo, hi)`` of
+        ``shard_range(global_batch, rank, world)``; a rank with an empty shard passes empty tensors and still takes part.
+        Afterwards every parameter's ``.grad`` holds the gradient of the global batch's loss (earlier ``.grad`` contents
+        are discarded).  Returns that loss (a 0-dim tensor, the same on every rank)."""
+        model = self.model
+        lo, hi = shard_range(int(global_batch), self.rank, self.world)
+        if pilots_local.shape[0] != hi - lo or truth_local.shape[0] != hi - lo:
+            raise ValueError(f"rank {self.rank} of {self.world} holds samples [{lo}, {hi}) of a {global_batch}-sample batch, "
+                             f"got {pilots_local.shape[0]} pilots and {truth_local.shape[0]} truths")
+        seed = self._seed()
+        model.zero_grad(set_to_none=True)
+        est = model(pilots_local, meta_local, sample_offset=lo, dropout_seed=seed)
+        truth = truth_local.to(est.device)
+        if tuple(truth.shape) != tuple(est.shape):
+            raise ValueError(f"truth_local has shape {tuple(truth.shape)}, the estimates {tuple(est.shape)}")
+        err = est - truth
+        count = 2 * int(global_batch) * est.shape[1] * est.shape[2]
+        loss = torch.cat([err.real, err.imag], 1).pow(2).sum() / max(count, 1)
+        loss.backward()
+        grads = [p.grad if p.grad is not None else torch.zeros_like(p) for p in self.params]
+        flat = torch.cat([g.reshape(-1) for g in grads] + [loss.detach().reshape(1).to(grads[0].dtype)])
+        if self.world > 1:
+            wire = flat.to(self._comm_device)
+            dist.all_reduce(wire, op=dist.ReduceOp.SUM, group=self.group)
+            flat = wire.to(flat.device)
+        off = 0
+        for p in self.params:
+            p.grad = flat[off:off + p.numel()].view_as(p)
+            off += p.numel()
+        return flat[off]

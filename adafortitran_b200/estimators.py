@@ -13,6 +13,7 @@ from __future__ import annotations
 import ctypes as C
 import logging
 import math
+import operator
 import os
 from typing import List, Optional, Tuple
 
@@ -153,7 +154,8 @@ class BaseFortiTranEstimator(nn.Module):
     every parameter (fp32 CUDA-core training path, reference default geometry): it applies the reference's dropout
     (``model_config.dropout``) in ``train()`` mode and none in ``eval()`` mode, and ``loss.backward()`` fills ``.grad``
     through ``aft_backward``.  Dropout masks are drawn from torch's default generator, so ``torch.manual_seed`` makes
-    runs reproducible.
+    runs reproducible; ``forward(..., sample_offset=, dropout_seed=)`` fixes them explicitly (data-parallel training,
+    :class:`adafortitran_b200.distributed.ShardedTrainer`).
     """
 
     trainable = False
@@ -419,7 +421,8 @@ class BaseFortiTranEstimator(nn.Module):
         return out
 
     # -- forward (fortitran.py:145-182) ---------------------------------------------------------
-    def forward(self, pilot_symbols: torch.Tensor, meta_data: Optional[Tuple] = None, gather=None) -> torch.Tensor:
+    def forward(self, pilot_symbols: torch.Tensor, meta_data: Optional[Tuple] = None, gather=None, *,
+                sample_offset: int = 0, dropout_seed: Optional[int] = None) -> torch.Tensor:
         """``pilot_symbols``: complex [batch, pilot_scs, pilot_symbols]; ``meta_data``: the reference 6-tuple
         ``(file_no, snr, delay_spread, max_dop_shift, pilot_freq, channel_type)`` (items 1..3 are used).
         Returns complex64 [batch, ofdm_scs, ofdm_symbols] on ``self.device``.
@@ -427,11 +430,22 @@ class BaseFortiTranEstimator(nn.Module):
         ``gather`` (keyword, optional; not part of the reference signature): a
         :class:`adafortitran_b200.distributed.PeerGather`; the kernel that writes the estimates then also stores them into
         every rank's gather buffer (fused all-gather over NVLink) and the returned tensor is this rank's slice of the
-        local gather buffer."""
+        local gather buffer.
+
+        ``sample_offset`` and ``dropout_seed`` (keywords, differentiable calls only): sample ``b`` of this call draws the
+        dropout masks of sample ``sample_offset + b`` of a larger batch, and ``dropout_seed`` (an integer in
+        ``[0, 2**64)``) replaces the seed otherwise drawn from torch's default generator.  Shards of one batch forwarded
+        with their offsets and one seed get exactly the masks of a single call over the whole batch.  A non-default
+        value on an inference call raises ``ValueError``."""
         precision = self._precision_code()
         batch, cond_in = self._check_call(pilot_symbols, meta_data, "cuda")
+        sample_offset = operator.index(sample_offset)
         if self.trainable and torch.is_grad_enabled():
-            return self._forward_differentiable(pilot_symbols, cond_in, batch, precision, gather)
+            return self._forward_differentiable(pilot_symbols, cond_in, batch, precision, gather, sample_offset,
+                                                dropout_seed)
+        if sample_offset != 0 or dropout_seed is not None:
+            raise ValueError("sample_offset / dropout_seed select dropout masks of a differentiable call: they have no "
+                             "meaning for inference (model.trainable = False or grad disabled)")
         self._ensure_handle()
         with torch.cuda.device(self.device):
             pilots = pilot_symbols.to(device=self.device, dtype=torch.complex64).contiguous()
@@ -464,7 +478,8 @@ class BaseFortiTranEstimator(nn.Module):
                     C.c_void_p(ws_ptr), ws.numel() - (ws_ptr - ws.data_ptr()), C.c_void_p(stream), C.byref(plan)))
         return out
 
-    def _forward_differentiable(self, pilot_symbols, cond_in, batch, precision, gather) -> torch.Tensor:
+    def _forward_differentiable(self, pilot_symbols, cond_in, batch, precision, gather, sample_offset,
+                                dropout_seed) -> torch.Tensor:
         if precision != _capi.AFT_FP32:
             raise ValueError("training (trainable = True with grad enabled) runs on the fp32 CUDA-core path only; "
                              "set model.precision = 'fp32' or run under torch.no_grad()")
@@ -474,6 +489,10 @@ class BaseFortiTranEstimator(nn.Module):
         if any(torch.is_tensor(t) and t.requires_grad for t in inputs):
             raise ValueError("gradients with respect to the pilots or the metadata are not computed: pass inputs that "
                              "do not require grad")
+        if dropout_seed is not None:
+            dropout_seed = operator.index(dropout_seed)
+            if not 0 <= dropout_seed < 2 ** 64:
+                raise ValueError(f"dropout_seed must be in [0, 2**64), got {dropout_seed}")
         self._ensure_handle()
         with torch.cuda.device(self.device):
             pilots = pilot_symbols.to(device=self.device, dtype=torch.complex64).contiguous()
@@ -481,9 +500,10 @@ class BaseFortiTranEstimator(nn.Module):
             if cond_in is not None:
                 cond = [t.to(device=self.device, dtype=torch.float32).reshape(-1).contiguous() for t in cond_in]
             p = float(self.model_config.dropout) if self.training else 0.0
-            seed = int(torch.randint(0, 2 ** 62, (), dtype=torch.int64).item())
+            if dropout_seed is None:
+                dropout_seed = int(torch.randint(0, 2 ** 62, (), dtype=torch.int64).item())
             named, _ = self._weight_tensors()
-            return _TrainForward.apply(self, pilots, cond, batch, p, seed, *[t for _, t in named])
+            return _TrainForward.apply(self, pilots, cond, batch, p, dropout_seed, sample_offset, *[t for _, t in named])
 
     def forward_host(self, pilot_symbols: torch.Tensor, meta_data: Optional[Tuple] = None,
                      out: Optional[torch.Tensor] = None, gather=None) -> torch.Tensor:
@@ -522,12 +542,12 @@ class BaseFortiTranEstimator(nn.Module):
 
 
 class _TrainForward(torch.autograd.Function):
-    """``aft_forward_train`` / ``aft_backward`` behind autograd.  The parameters are inputs of the Function (in the order
+    """``aft_forward_train_offset`` / ``aft_backward`` behind autograd.  The parameters are inputs of the Function (in the order
     of ``_weight_tensors``), so ``AccumulateGrad``, ``requires_grad=False``, hooks and version checks work as for any
     torch op; their gradients are views of the flat buffer ``aft_backward`` fills."""
 
     @staticmethod
-    def forward(ctx, model, pilots, cond, batch, p, seed, *params):
+    def forward(ctx, model, pilots, cond, batch, p, seed, sample0, *params):
         model._sync_weights()
         out = torch.empty((batch, *model.ofdm_size), dtype=torch.complex64, device=model.device)
         ws = None
@@ -540,8 +560,9 @@ class _TrainForward(torch.autograd.Function):
             ws_ptr = (ws.data_ptr() + 255) // 256 * 256
             vp = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
             stream = torch.cuda.current_stream(model.device).cuda_stream
-            _capi.check(lib.aft_forward_train(model._handle, vp(pilots), vp(cond[0]), vp(cond[1]), vp(cond[2]), vp(out),
-                                              batch, p, seed, C.c_void_p(ws_ptr), need, C.c_void_p(stream)))
+            _capi.check(lib.aft_forward_train_offset(model._handle, vp(pilots), vp(cond[0]), vp(cond[1]), vp(cond[2]),
+                                                     vp(out), batch, sample0, p, seed, C.c_void_p(ws_ptr), need,
+                                                     C.c_void_p(stream)))
         ctx.model, ctx.batch, ctx.ws = model, batch, ws
         ctx.save_for_backward(*params)
         return out
@@ -568,9 +589,9 @@ class _TrainForward(torch.autograd.Function):
         grads, off = [], 0
         for i, t in enumerate(params):
             k = t.numel()
-            grads.append(flat[off:off + k].view(t.shape).to(t.dtype) if ctx.needs_input_grad[6 + i] else None)
+            grads.append(flat[off:off + k].view(t.shape).to(t.dtype) if ctx.needs_input_grad[7 + i] else None)
             off += k
-        return (None, None, None, None, None, None, *grads)
+        return (None, None, None, None, None, None, None, *grads)
 
 
 class FortiTranEstimator(BaseFortiTranEstimator):

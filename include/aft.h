@@ -197,7 +197,7 @@ AFT_API int aft_profile_enable(AftHandle* h, int enable);
 AFT_API int aft_profile_read(AftHandle* h, double* ms, int64_t* launches);
 
 /* ---- Training (AFT_FP32 on CUDA cores, reference default geometry only) ----------------------------------------
- * A handle on any other geometry returns AFT_ERR_UNSUPPORTED from the four calls below.
+ * A handle on any other geometry returns AFT_ERR_UNSUPPORTED from the five calls below.
  *
  * Flat gradient layout: every parameter in torch layout without padding, in this order:
  *   pilot_upsampler w, b;  initial_enhancer w0 b0 w1 b1 w2 b2 w3 b3;  final_refiner w0 b0 .. w3 b3;
@@ -208,9 +208,12 @@ AFT_API int aft_profile_read(AftHandle* h, double* ms, int64_t* launches);
  * Dropout: nn.TransformerEncoderLayer's four sites (post-norm): 0 the attention probabilities, element index
  * (head*S + q)*S + k; 1 the out_proj output before the residual add, row*128 + col; 2 the FFN activation,
  * row*256 + col; 3 the linear2 output before the residual add, row*128 + col (row = token of the sequence).
- * Element i of sequence seq (= sample*2 + {0 re, 1 im}) in layer l at site s takes output word i & 3 of
- * Philox4x32-10 with key (seed & 0xffffffff, seed >> 32) and counter (i >> 2, seq, (l << 8) | s, 0), and is kept
- * iff that word >= floor(p * 2^32) (p as float, widened to double); kept values are scaled by 1 / (1 - p). */
+ * Element i of sequence seq = 2 * (sample0 + sample) + part (part 0 re, 1 im; sample = the index within the call,
+ * sample0 = the global index of the call's first sample, 0 for aft_forward_train) in layer l at site s takes output
+ * word i & 3 of Philox4x32-10 with key (seed & 0xffffffff, seed >> 32) and counter (i >> 2, seq, (l << 8) | s, 0),
+ * and is kept iff that word >= floor(p * 2^32) (p as float, widened to double); kept values are scaled by 1 / (1 - p).
+ * So a batch split into calls over consecutive sample ranges, each with its sample0 and the same seed, draws exactly
+ * the masks of one call over the whole batch. */
 
 /* Floats in the flat gradient buffer of aft_backward (0 on error). */
 AFT_API int64_t aft_param_count(const AftHandle* h);
@@ -223,6 +226,13 @@ AFT_API size_t aft_train_workspace_bytes(const AftHandle* h, int64_t batch);
 AFT_API int aft_forward_train(AftHandle* h, const void* pilots, const float* snr, const float* delay_spread,
                               const float* doppler, void* out, int64_t batch, float dropout, uint64_t seed,
                               void* workspace, size_t workspace_bytes, void* stream);
+/* aft_forward_train for samples sample0 .. sample0 + batch - 1 of a larger (e.g. data-parallel) batch: the dropout masks
+ * use the global sequence index (see "Dropout" above); aft_forward_train is the case sample0 = 0.  The sequence index is
+ * the 32-bit second counter word, so AFT_ERR_INVALID, with nothing launched, unless 0 <= sample0 and
+ * sample0 + batch <= 2^31.  aft_backward reads sample0 from the workspace with the seed and p. */
+AFT_API int aft_forward_train_offset(AftHandle* h, const void* pilots, const float* snr, const float* delay_spread,
+                                     const float* doppler, void* out, int64_t batch, int64_t sample0, float dropout,
+                                     uint64_t seed, void* workspace, size_t workspace_bytes, void* stream);
 /* Gradients of all parameters for grad_out = dL/d(out) (complex64 [batch, num_scs, num_symbols]: re = dL/dRe, im = dL/dIm).
  * Overwrites grads[aft_param_count(h)] (fp32, device).  Consumes the workspace of the aft_forward_train call it follows;
  * reads that call's header record back first (so it synchronises with `stream`) and returns AFT_ERR_INVALID when
