@@ -495,30 +495,48 @@ size_t aft_workspace_bytes(const AftHandle* h, int64_t batch, int precision) {
 
 namespace {
 
+bool misaligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) != 0; }
+
+// Destinations of a forward of `batch` > 0 samples, checked before anything is allocated, copied or launched, so that a
+// refused call leaves no work behind.  `has_out`: the chunks are computed into a device buffer `out` (the caller's, or
+// the staging lane of the host entry when `out` is NULL).  The fused tensor-core head stores whole rows by bulk copies;
+// a reference-grid row is 13,440 bytes, so a 16-byte aligned base keeps every row aligned.  The scatter kernel of the
+// other paths copies rows at any 8-byte offset, so gather buffers need an aligned base only.
+int check_dst(const AftHandle* h, bool has_out, const void* out, const AftGather* g, int64_t batch, int precision,
+              const char* fn) {
+  const bool fused = !h->generic && precision == AFT_BF16;
+  if (!has_out && !g) { set_error("%s: no destination (NULL out and no gather plan)", fn); return AFT_ERR_INVALID; }
+  if (!has_out && !fused) {
+    set_error("%s: this path needs a local `out` buffer (the scatter to the gather buffers reads it)", fn);
+    return AFT_ERR_INVALID;
+  }
+  if (fused && out && misaligned16(out)) { set_error("%s: out is not 16-byte aligned", fn); return AFT_ERR_INVALID; }
+  if (!g) return AFT_OK;
+  if (g->world < 1 || g->world > 8 || g->rank < 0 || g->rank >= g->world || g->rows_per_rank < 0 || g->row0 < 0) {
+    set_error("%s: bad gather plan (world %d, rank %d, rows_per_rank %lld, row0 %lld)", fn, g->world, g->rank,
+              (long long)g->rows_per_rank, (long long)g->row0);
+    return AFT_ERR_INVALID;
+  }
+  if (batch > g->rows_per_rank - g->row0) {
+    set_error("%s: rows [%lld, %lld) exceed rows_per_rank %lld", fn, (long long)g->row0, (long long)(g->row0 + batch),
+              (long long)g->rows_per_rank);
+    return AFT_ERR_INVALID;
+  }
+  for (int p = 0; p < g->world; ++p) {
+    if (!g->peer_out[p]) { set_error("%s: NULL gather buffer for rank %d", fn, p); return AFT_ERR_INVALID; }
+    if (misaligned16(g->peer_out[p])) { set_error("%s: gather buffer of rank %d is not 16-byte aligned", fn, p); return AFT_ERR_INVALID; }
+  }
+  return AFT_OK;
+}
+
 // destinations of the chunk that starts at local sample c0: the caller's buffer (if any) and, with a gather plan, this
-// rank's row range in every gather buffer
-int make_dst(const AftHandle* h, float2* out, const AftGather* g, int64_t c0, OutDst* dst) {
+// rank's row range in every gather buffer (checked by check_dst)
+void make_dst(const AftHandle* h, float2* out, const AftGather* g, int64_t c0, OutDst* dst) {
   dst->n = 0;
   if (out) dst->ptr[dst->n++] = out + c0 * h->pix;
-  if (g) {
-    if (g->world < 1 || g->world > 8 || g->rank < 0 || g->rank >= g->world || g->rows_per_rank < 0 || g->row0 < 0) {
-      set_error("gather plan: bad world / rank / rows_per_rank / row0");
-      return AFT_ERR_INVALID;
-    }
-    for (int p = 0; p < g->world; ++p) {
-      if (!g->peer_out[p]) { set_error("gather plan: NULL gather buffer for rank %d", p); return AFT_ERR_INVALID; }
+  if (g)
+    for (int p = 0; p < g->world; ++p)
       dst->ptr[dst->n++] = static_cast<float2*>(g->peer_out[p]) + (g->rank * g->rows_per_rank + g->row0 + c0) * h->pix;
-    }
-  }
-  if (dst->n == 0) { set_error("aft_forward: no destination (NULL out and no gather plan)"); return AFT_ERR_INVALID; }
-  // the estimates leave as 16-byte vectors / bulk copies of whole rows (a row is pix * 8 bytes: a multiple of 16 for the
-  // reference grid, so an aligned base keeps every row aligned)
-  for (int d = 0; d < dst->n; ++d)
-    if ((reinterpret_cast<uintptr_t>(dst->ptr[d]) & 15) != 0) {
-      set_error("aft_forward: output buffer %d is not 16-byte aligned", d);
-      return AFT_ERR_INVALID;
-    }
-  return AFT_OK;
 }
 
 int forward_impl(AftHandle* h, const void* pilots, const float* snr, const float* delay_spread, const float* doppler,
@@ -538,11 +556,6 @@ int aft_forward_gather(AftHandle* h, const void* pilots, const float* snr, const
                        void* out, int64_t batch, int precision, void* workspace, size_t workspace_bytes, void* stream,
                        const AftGather* gather) {
   if (!gather) { set_error("aft_forward_gather: NULL gather plan"); return AFT_ERR_INVALID; }
-  if (h && batch + gather->row0 > gather->rows_per_rank) {
-    set_error("aft_forward_gather: rows [%lld, %lld) exceed rows_per_rank %lld", (long long)gather->row0,
-              (long long)(gather->row0 + batch), (long long)gather->rows_per_rank);
-    return AFT_ERR_INVALID;
-  }
   return forward_impl(h, pilots, snr, delay_spread, doppler, out, batch, precision, workspace, workspace_bytes, stream, gather);
 }
 
@@ -565,7 +578,8 @@ int forward_impl(AftHandle* h, const void* pilots, const float* snr, const float
     }
   }
   const bool fused = !h->generic && precision == AFT_BF16;   // the tensor-core head stores to all destinations itself
-  if (!fused && !out) { set_error("aft_forward_gather: this path needs a local `out` buffer (the scatter to the peers reads it)"); return AFT_ERR_INVALID; }
+  int rc = check_dst(h, out != nullptr, out, gather, batch, precision, gather ? "aft_forward_gather" : "aft_forward");
+  if (rc != AFT_OK) return rc;
   const size_t need = aft_workspace_bytes(h, batch, precision);
   if (!workspace || workspace_bytes < need) {
     set_error("aft_forward: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
@@ -584,10 +598,8 @@ int forward_impl(AftHandle* h, const void* pilots, const float* snr, const float
     const float* s0 = h->cfg.adaptive ? snr + c0 : nullptr;
     const float* s1 = h->cfg.adaptive ? delay_spread + c0 : nullptr;
     const float* s2 = h->cfg.adaptive ? doppler + c0 : nullptr;
-    int rc;
     OutDst dst;
-    dst.n = 0;
-    if ((fused || gather) && (rc = make_dst(h, fused ? pout : nullptr, gather, c0, &dst)) != AFT_OK) return rc;
+    make_dst(h, fused ? pout : nullptr, gather, c0, &dst);
     if (h->generic) {
       rc = forward_chunk_generic(h, pin + c0 * h->P, s0, s1, s2, pout + c0 * h->pix, bc, static_cast<float*>(workspace), st, precision);
     } else if (precision == AFT_FP32) {
@@ -620,12 +632,16 @@ int aft_forward_host_gather(AftHandle* h, const void* pilots, const float* snr, 
   if (batch < 0) { set_error("aft_forward_host: negative batch"); return AFT_ERR_INVALID; }
   if (batch == 0) return AFT_OK;
   if (!pilots || (!out && !gather)) { set_error("aft_forward_host: NULL pilots / out"); return AFT_ERR_INVALID; }
-  if (gather && batch + gather->row0 > gather->rows_per_rank) { set_error("aft_forward_host_gather: rows exceed rows_per_rank"); return AFT_ERR_INVALID; }
+  if (precision != AFT_FP32 && precision != AFT_BF16) { set_error("aft_forward_host: bad precision %d", precision); return AFT_ERR_INVALID; }
+  if (!h->loaded) { set_error("aft_forward_host: weights not loaded (call aft_load_weights first)"); return AFT_ERR_STATE; }
   const bool ada = h->cfg.adaptive != 0;
   if (ada && (!snr || !delay_spread || !doppler)) {
     set_error("aft_forward_host: meta_data is required when channel adaptation is enabled");
     return AFT_ERR_INVALID;
   }
+  // every chunk is computed into a staging lane, so the plan is all there is left to refuse
+  int rc = check_dst(h, true, nullptr, gather, batch, precision, gather ? "aft_forward_host_gather" : "aft_forward_host");
+  if (rc != AFT_OK) return rc;
   int64_t hc = batch < kHostChunk ? batch : kHostChunk;
   if (h->generic && hc > chunk_for(h, precision)) hc = chunk_for(h, precision);
   const size_t in_bytes = (size_t)hc * (h->P * sizeof(float2) + 3 * sizeof(float));
@@ -666,25 +682,34 @@ int aft_forward_host_gather(AftHandle* h, const void* pilots, const float* snr, 
     }
     char* din = static_cast<char*>(ln.d_in);
     float* dmeta = reinterpret_cast<float*>(din + (size_t)ln.cap * h->P * sizeof(float2));
-    AFT_CUDA(cudaMemcpyAsync(din, hp + (size_t)c0 * h->P * sizeof(float2), (size_t)bc * h->P * sizeof(float2),
-                             cudaMemcpyHostToDevice, ln.stream));
-    if (ada) {
-      AFT_CUDA(cudaMemcpyAsync(dmeta, snr + c0, bc * sizeof(float), cudaMemcpyHostToDevice, ln.stream));
-      AFT_CUDA(cudaMemcpyAsync(dmeta + ln.cap, delay_spread + c0, bc * sizeof(float), cudaMemcpyHostToDevice, ln.stream));
-      AFT_CUDA(cudaMemcpyAsync(dmeta + 2 * ln.cap, doppler + c0, bc * sizeof(float), cudaMemcpyHostToDevice, ln.stream));
-    }
+    // from the first copy on, a failure breaks out of the loop: the lanes are synchronised below before the call
+    // returns, so no copy reads the caller's host buffers after it
+    auto copy = [&](void* dst, const void* src, size_t bytes, cudaMemcpyKind kind) {
+      const cudaError_t e = cudaMemcpyAsync(dst, src, bytes, kind, ln.stream);
+      if (e != cudaSuccess) { set_error("aft_forward_host: cudaMemcpyAsync failed: %s", cudaGetErrorString(e)); rc = AFT_ERR_CUDA; }
+      return rc == AFT_OK;
+    };
+    if (!copy(din, hp + (size_t)c0 * h->P * sizeof(float2), (size_t)bc * h->P * sizeof(float2), cudaMemcpyHostToDevice)) break;
+    if (ada && !(copy(dmeta, snr + c0, bc * sizeof(float), cudaMemcpyHostToDevice) &&
+                 copy(dmeta + ln.cap, delay_spread + c0, bc * sizeof(float), cudaMemcpyHostToDevice) &&
+                 copy(dmeta + 2 * ln.cap, doppler + c0, bc * sizeof(float), cudaMemcpyHostToDevice)))
+      break;
     AftGather gsub;
     if (gather) { gsub = *gather; gsub.row0 = gather->row0 + c0; }
-    const int rc = forward_impl(h, din, ada ? dmeta : nullptr, ada ? dmeta + ln.cap : nullptr, ada ? dmeta + 2 * ln.cap : nullptr,
-                                ln.d_out, bc, precision, ln.ws, ln.ws_bytes, ln.stream, gather ? &gsub : nullptr);
-    if (rc != AFT_OK) return rc;
-    if (out)
-      AFT_CUDA(cudaMemcpyAsync(ho + (size_t)c0 * h->pix * sizeof(float2), ln.d_out, (size_t)bc * h->pix * sizeof(float2),
-                               cudaMemcpyDeviceToHost, ln.stream));
+    rc = forward_impl(h, din, ada ? dmeta : nullptr, ada ? dmeta + ln.cap : nullptr, ada ? dmeta + 2 * ln.cap : nullptr,
+                      ln.d_out, bc, precision, ln.ws, ln.ws_bytes, ln.stream, gather ? &gsub : nullptr);
+    if (rc != AFT_OK) break;
+    if (out && !copy(ho + (size_t)c0 * h->pix * sizeof(float2), ln.d_out, (size_t)bc * h->pix * sizeof(float2), cudaMemcpyDeviceToHost))
+      break;
   }
-  AFT_CUDA(cudaStreamSynchronize(h->lanes[0].stream));
-  AFT_CUDA(cudaStreamSynchronize(h->lanes[1].stream));
-  return AFT_OK;
+  for (auto& ln : h->lanes) {
+    const cudaError_t e = cudaStreamSynchronize(ln.stream);
+    if (e != cudaSuccess && rc == AFT_OK) {
+      set_error("aft_forward_host: cudaStreamSynchronize failed: %s", cudaGetErrorString(e));
+      rc = AFT_ERR_CUDA;
+    }
+  }
+  return rc;
 }
 
 int aft_peer_alloc(size_t bytes, void** dev_ptr, void* handle64) {

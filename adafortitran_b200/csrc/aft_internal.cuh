@@ -80,7 +80,7 @@ struct HeadPack {
   ConvPack refine;
 };
 
-// Where the head stores the estimates of a chunk: up to 8 destinations (the caller's `out` and, for the fused
+// Where the head stores the estimates of a chunk: up to 9 destinations (the caller's `out` and, for the fused
 // all-gather of the multi-GPU evaluation path, this rank's row range inside every peer's gather buffer -- peer device
 // memory mapped into this process, written with plain 16-byte stores over NVLink).  ptr[d] addresses sample 0 of the chunk.
 struct OutDst {
@@ -144,7 +144,7 @@ bool launch_generic_head(const HeadPack& p, const float* h, const float* enh, fl
 
 // reduce.cu
 bool launch_error_sums(const float2* est, const float2* truth, int64_t count, double* sums, cudaStream_t st);
-// copies src[count] (complex64) to every destination of `dst` with 16-byte accesses (peer scatter of the non-fused paths)
+// copies src[count] (complex64) to every destination of `dst` (peer scatter of the non-fused paths), rows at any offset
 bool launch_scatter_rows(const float2* src, int64_t count, const OutDst& dst, cudaStream_t st);
 
 // ---------------------------------------------------------------------------------------------

@@ -33,12 +33,22 @@ error_sums_kernel(const float2* __restrict__ est, const float2* __restrict__ tru
   }
 }
 
-// src -> every destination, 16 bytes (two complex64) per access; count is even for every grid this library accepts
-// (an odd tail element is copied by thread 0)
-__global__ void __launch_bounds__(256) scatter_rows_kernel(const float2* __restrict__ src, int64_t count, OutDst dst) {
+// src -> every destination.  vec16 (the source and every destination 16-byte aligned): 16 bytes (two complex64) per
+// access, an odd tail element copied by thread 0.  Otherwise 8 bytes per access: a row is pix * 8 bytes, so on a grid
+// with odd pix a row at an odd offset is only 8-byte aligned.
+__global__ void __launch_bounds__(256)
+scatter_rows_kernel(const float2* __restrict__ src, int64_t count, OutDst dst, bool vec16) {
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  if (!vec16) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += stride) {
+      const float2 v = src[i];
+      for (int d = 0; d < dst.n; ++d) dst.ptr[d][i] = v;
+    }
+    return;
+  }
   const int64_t n4 = count >> 1;
   const float4* s4 = reinterpret_cast<const float4*>(src);
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
     const float4 v = s4[i];
     for (int d = 0; d < dst.n; ++d) reinterpret_cast<float4*>(dst.ptr[d])[i] = v;
   }
@@ -50,10 +60,12 @@ __global__ void __launch_bounds__(256) scatter_rows_kernel(const float2* __restr
 
 bool launch_scatter_rows(const float2* src, int64_t count, const OutDst& dst, cudaStream_t st) {
   if (dst.n <= 0 || count <= 0) return true;
+  bool vec16 = (reinterpret_cast<uintptr_t>(src) & 15) == 0;
+  for (int d = 0; d < dst.n; ++d) vec16 = vec16 && (reinterpret_cast<uintptr_t>(dst.ptr[d]) & 15) == 0;
   int64_t blocks = (count / 2 + 255) / 256;
   if (blocks > 148 * 4) blocks = 148 * 4;
   if (blocks < 1) blocks = 1;
-  scatter_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>(src, count, dst);
+  scatter_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>(src, count, dst, vec16);
   count_launch();
   return check_launch("scatter_rows_kernel");
 }

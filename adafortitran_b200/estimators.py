@@ -470,8 +470,12 @@ class BaseFortiTranEstimator(nn.Module):
                     C.c_void_p(ws_ptr), ws.numel() - (ws_ptr - ws.data_ptr()), C.c_void_p(stream)))
             else:
                 plan = gather.plan()
-                # fused tensor-core path: the head stores straight into the gather buffers; other paths stage in a local buffer
-                fused = precision == _capi.AFT_BF16 and not gather.force_staging
+                # fused tensor-core path (AFT_BF16 on the reference default geometry): the head stores straight into the
+                # gather buffers; every other path, the long-sequence bf16 path of other geometries included, computes
+                # into a local stage that the library then copies to the gather buffers
+                reference_geometry = (self.ofdm_size == (120, 14) and self.pilot_size == (12, 2)
+                                      and tuple(self.model_config.patch_size) == (3, 2))
+                fused = precision == _capi.AFT_BF16 and reference_geometry and not gather.force_staging
                 stage = None if fused else torch.empty((batch, *self.ofdm_size), dtype=torch.complex64, device=self.device)
                 _capi.check(_capi.lib().aft_forward_gather(
                     self._handle, vp(pilots), vp(cond[0]), vp(cond[1]), vp(cond[2]), vp(stage), batch, precision,

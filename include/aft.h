@@ -150,7 +150,14 @@ typedef struct AftGather {
   int64_t row0;           /* offset of this call's first sample inside the rank's shard (chunked callers)        */
 } AftGather;
 
-/* aft_forward with the fused all-gather.  `out` may be NULL (the estimates then only go to the gather buffers). */
+/* Every gather buffer peer_out[p], p < world, must be non-NULL with a 16-byte aligned base (cudaMalloc and CUDA IPC
+ * pointers always are); its rows may start at any offset, so rows_per_rank and row0 are free, including odd values on a
+ * grid with an odd number of points.  A call with batch > 0 checks the plan, the row range row0 + batch <= rows_per_rank
+ * and its destinations before it allocates, copies or launches anything, and returns AFT_ERR_INVALID with nothing
+ * enqueued when one is bad.  batch == 0 does nothing and returns AFT_OK. */
+
+/* aft_forward with the fused all-gather.  `out` may be NULL on the fused path (AFT_BF16 on the reference default grid;
+ * the estimates then only go to the gather buffers); every other path computes into `out` and copies from there. */
 AFT_API int aft_forward_gather(AftHandle* h, const void* pilots, const float* snr, const float* delay_spread,
                 const float* doppler, void* out, int64_t batch, int precision,
                 void* workspace, size_t workspace_bytes, void* stream, const AftGather* gather);

@@ -142,3 +142,26 @@ def test_error_sums_kernel(ada):
     assert abs(s[1] - np.sum(np.abs(b.astype(np.complex128)) ** 2)) / s[1] < 1e-6
     # the reference's reported metric from these sums
     assert abs(10 * np.log10(s[0] / a.size) - O.mse_db_reference(a, b)) < 1e-4
+    # Grid edges of the capped grid (148 * 8 blocks of 256 threads, grid-stride): one element, a partial block, one
+    # element past a block, one element past one pass (303,105), and 4096 estimates + 3.  Magnitudes 1e-3 .. 1e3, every
+    # fifth element with est == truth, sums prefilled (the call accumulates).  Each term is formed in fp32 and added in
+    # fp64: a non-negative term is off by at most 4 * 2^-24, so the sums are within 3e-7 of fp64 sums of the same inputs.
+    lib = _capi.lib()
+    for n in (1, 255, 257, 148 * 8 * 256 + 1, 4096 * 1680 + 3):
+        mag = 10.0 ** rng.uniform(-3, 3, size=(2, n))
+        a = (mag[0] * (rng.standard_normal(n) + 1j * rng.standard_normal(n))).astype(np.complex64)
+        b = (mag[1] * (rng.standard_normal(n) + 1j * rng.standard_normal(n))).astype(np.complex64)
+        a[3::5] = b[3::5]
+        ref = np.array([np.sum(np.abs(a.astype(np.complex128) - b) ** 2), np.sum(np.abs(b.astype(np.complex128)) ** 2)])
+        pre = np.array([0.375, 0.625]) * ref
+        ta, tb = torch.from_numpy(a).cuda(), torch.from_numpy(b).cuda()
+        sums = torch.from_numpy(pre.copy()).cuda()
+        _capi.check(lib.aft_error_sums(C.c_void_p(ta.data_ptr()), C.c_void_p(tb.data_ptr()), n,
+                                       C.c_void_p(sums.data_ptr()), C.c_void_p(st)))
+        err = np.abs(sums.cpu().numpy() - (pre + ref))
+        assert (err <= 3e-7 * ref).all(), (n, err / ref)
+    kept, before = sums.cpu().numpy(), lib.aft_launch_count()     # count 0: nothing launched, sums untouched
+    _capi.check(lib.aft_error_sums(C.c_void_p(ta.data_ptr()), C.c_void_p(tb.data_ptr()), 0, C.c_void_p(sums.data_ptr()),
+                                   C.c_void_p(st)))
+    assert lib.aft_launch_count() == before
+    assert np.array_equal(sums.cpu().numpy(), kept)

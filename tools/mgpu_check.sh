@@ -1,10 +1,9 @@
 #!/bin/bash
-# GPU box (N GPUs): fused all-gather check + the sharded bench at 8192 estimates per rank (the per-rank load of the 8-GPU run).
+# N GPUs: the sharded bench at 8192 estimates per rank (the per-rank load of the 8-GPU run).
 set -u
 N=${1:-2}
 mkdir -p gpurun_out
 unset AFT_ENCODER AFT_B200_LIB
-timeout 300 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port 29511 tools/gather_check.py 2048 bf16 2>&1 | grep -v "^\*\|OMP_NUM\|^$" | tail -3
 timeout 400 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port 29512 bench.py --gpus $N --global-batch $((8192*N)) --steps 6 --warmup 3 --no-cpu-baseline > gpurun_out/mgpu_${N}.json 2> gpurun_out/mgpu_${N}.err
 python - <<PY
 import json
