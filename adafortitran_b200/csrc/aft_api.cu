@@ -776,6 +776,30 @@ int aft_linear_forward(const float* weight, const float* bias, const float* x, f
   return launch_linear(weight, bias, x, y, batch, in_dim, out_dim, static_cast<cudaStream_t>(stream)) ? AFT_OK : AFT_ERR_CUDA;
 }
 
+size_t aft_linear_backward_workspace_bytes(int64_t batch, int32_t in_dim, int32_t out_dim) {
+  if (batch < 0 || in_dim <= 0 || out_dim <= 0 || in_dim > 4096) {
+    set_error("aft_linear_backward_workspace_bytes: bad shape (batch >= 0, 0 < in_dim <= 4096, out_dim > 0)");
+    return 0;
+  }
+  return linear_backward_workspace_bytes(batch, in_dim, out_dim);
+}
+
+int aft_linear_backward(const float* weight, const float* x, const float* grad_y, float* grad_w, float* grad_b, float* grad_x,
+                        int64_t batch, int32_t in_dim, int32_t out_dim, void* workspace, size_t workspace_bytes, void* stream) {
+  if (batch < 0 || in_dim <= 0 || out_dim <= 0 || !weight || !grad_w || !grad_b || (batch > 0 && (!x || !grad_y))) {
+    set_error("aft_linear_backward: bad argument");
+    return AFT_ERR_INVALID;
+  }
+  if (in_dim > 4096) { set_error("aft_linear_backward: in_dim %d not supported (<= 4096)", in_dim); return AFT_ERR_INVALID; }
+  const size_t need = linear_backward_workspace_bytes(batch, in_dim, out_dim);
+  if (!workspace || workspace_bytes < need) {
+    set_error("aft_linear_backward: workspace too small (%zu < %zu bytes)", workspace_bytes, need);
+    return AFT_ERR_WORKSPACE;
+  }
+  return launch_linear_backward(weight, x, grad_y, grad_w, grad_b, grad_x, batch, in_dim, out_dim, workspace,
+                                static_cast<cudaStream_t>(stream)) ? AFT_OK : AFT_ERR_CUDA;
+}
+
 int aft_profile_enable(AftHandle* h, int enable) {
   if (!h) { set_error("aft_profile_enable: NULL handle"); return AFT_ERR_INVALID; }
   h->profile = enable != 0;

@@ -132,6 +132,9 @@ bool launch_attn_f32(const float* qkv, float* out, int64_t nseq, cudaStream_t st
 // aux.cu : "next" rows N2 / N3 -- pilot extraction from the sparse LS grid, LinearEstimator
 bool launch_extract_pilots(const float2* grid, float2* pilots, int32_t* counts, int64_t batch, int cells, int expected, cudaStream_t st);
 bool launch_linear(const float* w, const float* bias, const float* x, float* y, int64_t batch, int in_dim, int out_dim, cudaStream_t st);
+size_t linear_backward_workspace_bytes(int64_t batch, int in_dim, int out_dim);   // >= 256
+bool launch_linear_backward(const float* w, const float* x, const float* gy, float* grad_w, float* grad_b, float* grad_x,
+                            int64_t batch, int in_dim, int out_dim, void* workspace, cudaStream_t st);
 
 // generic_f32.cu : AFT_FP32 path for non-default grids (activations in global memory, runtime extents)
 size_t generic_front_scratch_floats(int64_t nsamples, int P, int pix, int S);

@@ -189,7 +189,244 @@ linear_kernel(const float* __restrict__ w, const float* __restrict__ bias, const
   }
 }
 
+// LinearEstimator backward: the three products of y = W x + b, all C[m][n] = sum_r A[r][m] B[r][n] in one kernel family.
+//   kXgrad false: C[o][c] = sum_b gy[b][o] [x | 1][b][c]  -> grad_w[o][k] (c < in_dim) and grad_b[o] (c == in_dim)
+//   kXgrad true : C[b][k] = sum_o gy[b][o] W[o][k]        -> grad_x
+// A CTA owns a slab of kBwdTileM rows of C and TX * 4 of its columns; a thread owns 4 x 4 elements.  The reduction index r
+// runs in groups of kBwdGroup staged in shared memory (the next group is loaded into registers while the current one is
+// computed).  Each group's 32 products are summed in fp32 and the group sums are added in fp64, so the error does not
+// grow with the length of the sum (10^6 samples, or out_dim = 45864 for grad_x).  The weight gradient splits the batch
+// over blockIdx.z into contiguous ranges of whole groups (linear_bwd_plan); with more than one range every CTA writes an
+// fp32 partial of its tile and linear_bwd_reduce_kernel adds the partials in range order in fp64.  No atomics anywhere:
+// the same inputs give bit-identical gradients.  kVec: 16-byte global loads (the reference shape, 16-byte aligned gy,
+// x and W, out_dim % 4 == 0); otherwise element loads with any alignment and any extents.
+constexpr int kBwdTileM = 128, kBwdGroup = 32;
+
+template <bool kXgrad, int TX, bool kVec>
+__global__ void __launch_bounds__(32 * TX)
+linear_bwd_kernel(const float* __restrict__ gy, const float* __restrict__ bop, float* __restrict__ c0, float* __restrict__ c1,
+                  int64_t batch, int in_dim, int out_dim, int64_t range) {
+  constexpr int kThreads = 32 * TX, kTileN = 4 * TX, G = kBwdGroup;
+  constexpr int kA4 = (G * kBwdTileM / 4 + kThreads - 1) / kThreads;   // 16-byte A loads per thread and group
+  constexpr int kA1 = (G * kBwdTileM + kThreads - 1) / kThreads;       // element A loads
+  __shared__ __align__(16) float As[G][kBwdTileM + 4];
+  __shared__ __align__(16) float Bs[G][kTileN];
+  const int tid = threadIdx.x, tx = tid % TX, ty = tid / TX;
+  const int64_t M = kXgrad ? batch : out_dim, R = kXgrad ? (int64_t)out_dim : batch;
+  const int N = kXgrad ? in_dim : in_dim + 1;
+  const int64_t m0 = (int64_t)blockIdx.x * kBwdTileM;
+  const int n0 = blockIdx.y * kTileN;
+  const int64_t r_begin = kXgrad ? 0 : (int64_t)blockIdx.z * range;
+  const int64_t r_end = kXgrad ? R : (r_begin + range < R ? r_begin + range : R);
+
+  // A[r][m]: gy[r][m] (weight gradient) or gy[m][r] (input gradient).  B[r][n]: [x | 1][r][n] or W[r][n].  Out of range: 0.
+  auto a_at = [&](int64_t r, int64_t m) -> float {
+    if (r >= r_end || m >= M) return 0.f;
+    return kXgrad ? gy[m * out_dim + r] : gy[r * out_dim + m];
+  };
+  auto b_at = [&](int64_t r, int n) -> float {
+    if (r >= r_end || n >= N) return 0.f;
+    if (!kXgrad && n == in_dim) return 1.f;
+    return bop[r * in_dim + n];
+  };
+  float4 pa4[kVec ? kA4 : 1], pb4;
+  float pa1[kVec ? 1 : kA1], pb1[kVec ? 1 : 4];
+  auto load = [&](int64_t r0) {
+    if (kVec) {
+#pragma unroll
+      for (int i = 0; i < kA4; ++i) {
+        const int idx = tid + i * kThreads;
+        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (idx < G * kBwdTileM / 4) {
+          // weight gradient: 4 consecutive outputs of one sample; input gradient: 4 consecutive outputs of one sample
+          // (transposed into As on the store).  out_dim % 4 == 0, so a vector is either all in range or all out.
+          const int64_t r = kXgrad ? r0 + 4 * (idx % (G / 4)) : r0 + idx / (kBwdTileM / 4);
+          const int64_t m = kXgrad ? m0 + idx / (G / 4) : m0 + 4 * (idx % (kBwdTileM / 4));
+          if (r < r_end && m < M) v = *reinterpret_cast<const float4*>(kXgrad ? gy + m * out_dim + r : gy + r * out_dim + m);
+        }
+        pa4[i] = v;
+      }
+      const int64_t r = r0 + ty;
+      const int n = n0 + 4 * tx;   // in_dim % 4 == 0: a vector of B is all columns < in_dim or all >= in_dim
+      pb4 = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (r < r_end && n < in_dim) pb4 = *reinterpret_cast<const float4*>(bop + r * in_dim + n);
+      else if (r < r_end && !kXgrad && n == in_dim) pb4.x = 1.f;
+    } else {
+#pragma unroll
+      for (int i = 0; i < kA1; ++i) {
+        const int idx = tid + i * kThreads;
+        // consecutive threads read consecutive addresses: m fastest (weight gradient), r fastest (input gradient)
+        pa1[i] = idx >= G * kBwdTileM ? 0.f
+                 : kXgrad ? a_at(r0 + idx % G, m0 + idx / G) : a_at(r0 + idx / kBwdTileM, m0 + idx % kBwdTileM);
+      }
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const int idx = tid + i * kThreads;
+        pb1[i] = b_at(r0 + idx / kTileN, n0 + idx % kTileN);
+      }
+    }
+  };
+  auto store = [&]() {
+    if (kVec) {
+#pragma unroll
+      for (int i = 0; i < kA4; ++i) {
+        const int idx = tid + i * kThreads;
+        if (idx >= G * kBwdTileM / 4) continue;
+        if (kXgrad) {
+          const int r = 4 * (idx % (G / 4)), m = idx / (G / 4);
+          As[r][m] = pa4[i].x; As[r + 1][m] = pa4[i].y; As[r + 2][m] = pa4[i].z; As[r + 3][m] = pa4[i].w;
+        } else {
+          *reinterpret_cast<float4*>(&As[idx / (kBwdTileM / 4)][4 * (idx % (kBwdTileM / 4))]) = pa4[i];
+        }
+      }
+      *reinterpret_cast<float4*>(&Bs[ty][4 * tx]) = pb4;
+    } else {
+#pragma unroll
+      for (int i = 0; i < kA1; ++i) {
+        const int idx = tid + i * kThreads;
+        if (idx >= G * kBwdTileM) continue;
+        if (kXgrad) As[idx % G][idx / G] = pa1[i];
+        else As[idx / kBwdTileM][idx % kBwdTileM] = pa1[i];
+      }
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const int idx = tid + i * kThreads;
+        Bs[idx / kTileN][idx % kTileN] = pb1[i];
+      }
+    }
+  };
+
+  double dacc[4][4];
+#pragma unroll
+  for (int i = 0; i < 4; ++i)
+#pragma unroll
+    for (int j = 0; j < 4; ++j) dacc[i][j] = 0.0;
+  if (r_begin < r_end) load(r_begin);
+  for (int64_t r0 = r_begin; r0 < r_end; r0 += G) {
+    store();
+    __syncthreads();
+    if (r0 + G < r_end) load(r0 + G);
+    float acc[4][4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+      for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
+#pragma unroll 8
+    for (int r = 0; r < G; ++r) {
+      const float4 a = *reinterpret_cast<const float4*>(&As[r][4 * ty]);
+      const float4 b = *reinterpret_cast<const float4*>(&Bs[r][4 * tx]);
+      const float av[4] = {a.x, a.y, a.z, a.w}, bv[4] = {b.x, b.y, b.z, b.w};
+#pragma unroll
+      for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(av[i], bv[j], acc[i][j]);
+    }
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+      for (int j = 0; j < 4; ++j) dacc[i][j] += acc[i][j];
+    __syncthreads();
+  }
+
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int64_t m = m0 + 4 * ty + i;
+    if (m >= M) continue;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const int n = n0 + 4 * tx + j;
+      if (n >= N) continue;
+      const float v = (float)dacc[i][j];
+      if (kXgrad) c0[m * in_dim + n] = v;
+      else if (gridDim.z > 1) c0[((int64_t)blockIdx.z * M + m) * N + n] = v;   // partial of batch range z, [z][o][in_dim + 1]
+      else if (n < in_dim) c0[m * in_dim + n] = v;
+      else c1[m] = v;
+    }
+  }
+}
+
+// grad_w / grad_b from the partials of the nz batch ranges, summed in range order in fp64
+__global__ void __launch_bounds__(256)
+linear_bwd_reduce_kernel(const float* __restrict__ part, int nz, int64_t count, int in_dim, float* __restrict__ grad_w,
+                         float* __restrict__ grad_b) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  double s = 0.0;
+  for (int z = 0; z < nz; ++z) s += part[z * count + i];
+  const int64_t o = i / (in_dim + 1);
+  const int c = (int)(i - o * (in_dim + 1));
+  if (c < in_dim) grad_w[o * in_dim + c] = (float)s;
+  else grad_b[o] = (float)s;
+}
+
+// Split of the batch for the weight gradient, a function of the shape only (so the workspace size is too): enough
+// batch ranges for ~4 CTAs per SM, at most 64, each a whole number of groups; no split once the tiles alone fill that.
+struct LinearBwdPlan {
+  int64_t nz, range;
+};
+LinearBwdPlan linear_bwd_plan(int64_t batch, int in_dim, int out_dim) {
+  constexpr int64_t kTarget = 4 * 148, kMaxSplit = 64;
+  const int64_t tiles = (out_dim + kBwdTileM - 1) / kBwdTileM * ((in_dim + 1 + 31) / 32);
+  const int64_t groups = (batch + kBwdGroup - 1) / kBwdGroup;
+  int64_t nz = tiles >= kTarget ? 1 : (kTarget + tiles - 1) / tiles;
+  if (nz > kMaxSplit) nz = kMaxSplit;
+  if (nz > groups) nz = groups;
+  if (nz < 1) nz = 1;
+  const int64_t per = groups > 0 ? (groups + nz - 1) / nz : 1;   // groups per range
+  return {groups > 0 ? (groups + per - 1) / per : 1, per * kBwdGroup};
+}
+
 }  // namespace
+
+size_t linear_backward_workspace_bytes(int64_t batch, int in_dim, int out_dim) {
+  const LinearBwdPlan p = linear_bwd_plan(batch, in_dim, out_dim);
+  const size_t part = p.nz > 1 ? (size_t)p.nz * out_dim * (in_dim + 1) * sizeof(float) : 0;
+  return part > 256 ? part : 256;
+}
+
+bool launch_linear_backward(const float* w, const float* x, const float* gy, float* grad_w, float* grad_b, float* grad_x,
+                            int64_t batch, int in_dim, int out_dim, void* workspace, cudaStream_t st) {
+  if (batch == 0) {   // empty sums: zero gradients
+    if (cudaMemsetAsync(grad_w, 0, (size_t)out_dim * in_dim * sizeof(float), st) != cudaSuccess ||
+        cudaMemsetAsync(grad_b, 0, (size_t)out_dim * sizeof(float), st) != cudaSuccess) {
+      set_error("aft_linear_backward: cudaMemsetAsync failed");
+      return false;
+    }
+    return true;
+  }
+  auto a16 = [](const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; };
+  const bool ref = in_dim == 24 && out_dim % 4 == 0 && a16(gy);   // the reference shape: 16-byte loads
+  const LinearBwdPlan p = linear_bwd_plan(batch, in_dim, out_dim);
+  float* part = p.nz > 1 ? static_cast<float*>(workspace) : grad_w;
+  // columns of [x | 1]: 28 per CTA on the fast path (24 + bias + 3 zero), 32 otherwise; one column tile for in_dim = 24
+  // either way, so the split does not depend on the path
+  const dim3 gw((unsigned)((out_dim + kBwdTileM - 1) / kBwdTileM), (unsigned)((in_dim + 1 + 31) / 32), (unsigned)p.nz);
+  if (ref && a16(x)) {
+    linear_bwd_kernel<false, 7, true><<<gw, 32 * 7, 0, st>>>(gy, x, part, grad_b, batch, in_dim, out_dim, p.range);
+  } else {
+    linear_bwd_kernel<false, 8, false><<<gw, 32 * 8, 0, st>>>(gy, x, part, grad_b, batch, in_dim, out_dim, p.range);
+  }
+  count_launch();
+  if (!check_launch("linear_bwd_kernel")) return false;
+  if (p.nz > 1) {
+    const int64_t count = (int64_t)out_dim * (in_dim + 1);
+    linear_bwd_reduce_kernel<<<(unsigned)((count + 255) / 256), 256, 0, st>>>(part, (int)p.nz, count, in_dim, grad_w, grad_b);
+    count_launch();
+    if (!check_launch("linear_bwd_reduce_kernel")) return false;
+  }
+  if (grad_x) {
+    const unsigned rows = (unsigned)((batch + kBwdTileM - 1) / kBwdTileM);
+    if (ref && a16(w)) {
+      linear_bwd_kernel<true, 6, true><<<dim3(rows, 1), 32 * 6, 0, st>>>(gy, w, grad_x, nullptr, batch, in_dim, out_dim, 0);
+    } else {
+      linear_bwd_kernel<true, 8, false><<<dim3(rows, (unsigned)((in_dim + 31) / 32)), 32 * 8, 0, st>>>(gy, w, grad_x, nullptr, batch,
+                                                                                                     in_dim, out_dim, 0);
+    }
+    count_launch();
+    if (!check_launch("linear_bwd_kernel")) return false;
+  }
+  return true;
+}
 
 bool launch_extract_pilots(const float2* grid, float2* pilots, int32_t* counts, int64_t batch, int cells, int expected, cudaStream_t st) {
   if (batch <= 0) return true;

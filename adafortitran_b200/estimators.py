@@ -615,7 +615,14 @@ class AdaFortiTranEstimator(BaseFortiTranEstimator):
 class LinearEstimator(nn.Module):
     """Learned linear estimator ``h_hat = W h_pilot + b`` (reference src/models/linear.py:15-107): same constructor,
     attributes, ``state_dict`` keys (``linear.weight`` [out, in], ``linear.bias``) and shape check; the product runs in
-    ``aft_linear_forward``.  Like the reference's ``nn.Linear`` it is a real-valued map: complex input is rejected."""
+    ``aft_linear_forward``.  Like the reference's ``nn.Linear`` it is a real-valued map: complex input is rejected.
+
+    ``trainable`` (default ``False``): with ``True``, a ``forward`` with grad enabled is differentiable, in ``train()`` and
+    ``eval()`` mode alike (the model has no dropout): ``loss.backward()`` fills ``.grad`` of the weight, the bias and, when
+    it requires grad, the input through ``aft_linear_backward``.  The output equals the ``no_grad`` output bit for bit, and
+    gradients come back in the dtype of the tensor they belong to."""
+
+    trainable = False
 
     def __init__(self, system_config: SystemConfig, model_config: ModelConfig) -> None:
         super().__init__()
@@ -644,20 +651,65 @@ class LinearEstimator(nn.Module):
         if device.type != "cuda" or self.linear.bias.device != device:
             raise RuntimeError(f"adafortitran_b200 has no CPU fallback: the parameters live on '{device}', move the model "
                                "to a CUDA device (.to('cuda'))")
+        if self.trainable and torch.is_grad_enabled():
+            out = _LinearTrain.apply(x, self.linear.weight, self.linear.bias)
+            return out.reshape(-1, self.ofdm_size[0], self.ofdm_size[1])
         if self.training and torch.is_grad_enabled():
             raise RuntimeError("adafortitran_b200 is inference-only: call model.eval() or wrap the call in torch.no_grad()")
-        # the kernel reads fp32, contiguous parameters: convert (no-op for the reference's own layout) instead of
-        # handing over pointers to anything else
-        w = self.linear.weight.detach().to(torch.float32).contiguous()
-        b = self.linear.bias.detach().to(torch.float32).contiguous()
-        xin = x.to(device=device, dtype=torch.float32).reshape(x.size(0), self.linear.in_features).contiguous()
-        out = torch.empty((x.size(0), self.linear.out_features), dtype=torch.float32, device=device)
-        with torch.cuda.device(device):
-            stream = torch.cuda.current_stream(device).cuda_stream
-            _capi.check(_capi.lib().aft_linear_forward(
-                C.c_void_p(w.data_ptr()), C.c_void_p(b.data_ptr()), C.c_void_p(xin.data_ptr()),
-                C.c_void_p(out.data_ptr()), x.size(0), self.linear.in_features, self.linear.out_features, C.c_void_p(stream)))
+        out, _, _ = _linear_forward(x, self.linear.weight, self.linear.bias)
         return out.reshape(-1, self.ofdm_size[0], self.ofdm_size[1])
 
     def __repr__(self) -> str:
         return f"LinearEstimator(\n  ofdm_size={self.ofdm_size},\n  pilot_size={self.pilot_size},\n  device={self.device}\n)"
+
+
+def _linear_forward(x: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor):
+    """``aft_linear_forward`` on fp32, contiguous copies of the operands (no-ops for the reference's own layout) instead of
+    pointers to anything else.  Returns the output [batch, out] and the fp32 weight and input it was computed from."""
+    device = weight.device
+    w = weight.detach().to(torch.float32).contiguous()
+    b = bias.detach().to(torch.float32).contiguous()
+    xin = x.detach().to(device=device, dtype=torch.float32).reshape(x.size(0), w.shape[1]).contiguous()
+    out = torch.empty((x.size(0), w.shape[0]), dtype=torch.float32, device=device)
+    with torch.cuda.device(device):
+        stream = torch.cuda.current_stream(device).cuda_stream
+        _capi.check(_capi.lib().aft_linear_forward(
+            C.c_void_p(w.data_ptr()), C.c_void_p(b.data_ptr()), C.c_void_p(xin.data_ptr()),
+            C.c_void_p(out.data_ptr()), x.size(0), w.shape[1], w.shape[0], C.c_void_p(stream)))
+    return out, w, xin
+
+
+class _LinearTrain(torch.autograd.Function):
+    """``aft_linear_forward`` / ``aft_linear_backward`` behind autograd for :class:`LinearEstimator` with
+    ``trainable = True``.  The input gradient is computed only when the input needs one."""
+
+    @staticmethod
+    def forward(ctx, x, weight, bias):
+        out, w, xin = _linear_forward(x, weight, bias)
+        ctx.save_for_backward(w, xin)
+        ctx.x_meta = (x.shape, x.dtype, x.device)
+        ctx.param_dtypes = (weight.dtype, bias.dtype)
+        return out
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        w, xin = ctx.saved_tensors
+        (x_shape, x_dtype, x_device), device = ctx.x_meta, w.device
+        batch, (out_dim, in_dim) = xin.shape[0], w.shape
+        gy = grad_out.to(device=device, dtype=torch.float32).contiguous()
+        grad_w = torch.empty((out_dim, in_dim), dtype=torch.float32, device=device)
+        grad_b = torch.empty(out_dim, dtype=torch.float32, device=device)
+        grad_x = torch.empty((batch, in_dim), dtype=torch.float32, device=device) if ctx.needs_input_grad[0] else None
+        lib = _capi.lib()
+        need = lib.aft_linear_backward_workspace_bytes(batch, in_dim, out_dim)
+        if need == 0:
+            _capi.check(_capi.AFT_ERR_INVALID)
+        ws = torch.empty(need, dtype=torch.uint8, device=device)
+        vp = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        with torch.cuda.device(device):
+            stream = torch.cuda.current_stream(device).cuda_stream
+            _capi.check(lib.aft_linear_backward(vp(w), vp(xin), vp(gy), vp(grad_w), vp(grad_b), vp(grad_x), batch, in_dim,
+                                                out_dim, vp(ws), need, C.c_void_p(stream)))
+        (w_dtype, b_dtype), (_, need_w, need_b) = ctx.param_dtypes, ctx.needs_input_grad
+        return (grad_x.reshape(x_shape).to(device=x_device, dtype=x_dtype) if grad_x is not None else None,
+                grad_w.to(w_dtype) if need_w else None, grad_b.to(b_dtype) if need_b else None)

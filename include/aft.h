@@ -193,6 +193,25 @@ AFT_API int aft_extract_pilots(const void* ls_grid, void* pilots, int32_t* count
 AFT_API int aft_linear_forward(const float* weight, const float* bias, const float* x, float* y, int64_t batch,
                                int32_t in_dim, int32_t out_dim, void* stream);
 
+/* Bytes of device scratch aft_linear_backward needs for this shape (at least 256; 0 on error: batch < 0, in_dim outside
+ * 1..4096, out_dim <= 0).  The weight gradient splits the batch into at most 64 contiguous ranges; this is room for their
+ * fp32 partial sums. */
+AFT_API size_t aft_linear_backward_workspace_bytes(int64_t batch, int32_t in_dim, int32_t out_dim);
+
+/* Backward of aft_linear_forward (training LinearEstimator), fp32, device pointers:
+ *   grad_w[o, k] = sum_b grad_y[b, o] x[b, k]     [out_dim, in_dim]
+ *   grad_b[o]    = sum_b grad_y[b, o]             [out_dim]
+ *   grad_x[b, k] = sum_o grad_y[b, o] W[o, k]     [batch, in_dim]; skipped when grad_x is NULL
+ * grad_w, grad_b and grad_x are overwritten, not accumulated; batch == 0 writes zero grad_w / grad_b.  Sums are taken in
+ * fp32 over groups of 32 terms and in fp64 across groups, in a fixed order without atomics: the same inputs give
+ * bit-identical gradients.  Same shapes as aft_linear_forward (in_dim <= 4096, any out_dim) and any alignment.
+ * Asynchronous on `stream`; no allocation, no host synchronisation.  AFT_ERR_INVALID (NULL weight / grad_w / grad_b, NULL
+ * x / grad_y with batch > 0, negative or zero sizes, in_dim > 4096) or AFT_ERR_WORKSPACE (workspace NULL or smaller than
+ * aft_linear_backward_workspace_bytes) with nothing launched. */
+AFT_API int aft_linear_backward(const float* weight, const float* x, const float* grad_y, float* grad_w, float* grad_b,
+                                float* grad_x, int64_t batch, int32_t in_dim, int32_t out_dim, void* workspace,
+                                size_t workspace_bytes, void* stream);
+
 /* Number of kernel launches issued by this library on the calling process since load (for bench.py). */
 AFT_API int64_t aft_launch_count(void);
 
