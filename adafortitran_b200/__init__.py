@@ -3,6 +3,7 @@
 Public surface (mirrors the reference's ``src.models`` / ``src.config``):
     FortiTranEstimator, AdaFortiTranEstimator, BaseFortiTranEstimator, LinearEstimator
     data.extract_values, data.extract_pilots, data.MatDataset, data.collate_on_device   (input side, row N2)
+    data.SyntheticChannels                                                             (data generated on the GPU)
     SystemConfig, ModelConfig, load_config
 """
 from .config import ConfigLoader, ModelConfig, OFDMParams, PilotParams, SystemConfig, load_config

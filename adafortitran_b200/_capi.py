@@ -83,6 +83,8 @@ EXPORTS = {
     "aft_linear_backward_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int32, C.c_int32]),
     "aft_linear_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
                                       C.c_int32, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "aft_synthetic_channels": (C.c_int, [C.POINTER(AftConfig), C.c_uint64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p,
+                                         C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "aft_launch_count": (C.c_int64, []),
     "aft_profile_enable": (C.c_int, [C.c_void_p, C.c_int]),
     "aft_profile_read": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int64)]),

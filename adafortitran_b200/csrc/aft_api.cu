@@ -800,6 +800,39 @@ int aft_linear_backward(const float* weight, const float* x, const float* grad_y
                                 static_cast<cudaStream_t>(stream)) ? AFT_OK : AFT_ERR_CUDA;
 }
 
+int aft_synthetic_channels(const AftConfig* cfg, uint64_t seed, int64_t sample0, int64_t batch, float* snr, float* delay_spread,
+                           float* doppler, int32_t draw_conditions, void* pilots, void* truth, void* stream) {
+  if (!cfg) { set_error("aft_synthetic_channels: NULL config"); return AFT_ERR_INVALID; }
+  if (batch < 0 || sample0 < 0 || batch > INT64_MAX - sample0) {
+    set_error("aft_synthetic_channels: samples [%lld, %lld + %lld) outside [0, 2^63)", (long long)sample0, (long long)sample0,
+              (long long)batch);
+    return AFT_ERR_INVALID;
+  }
+  const AftConfig& c = *cfg;
+  if (c.num_scs <= 0 || c.num_symbols <= 0 || c.pilot_scs <= 0 || c.pilot_symbols <= 0 || c.pilot_scs > c.num_scs ||
+      c.pilot_symbols > 2 || c.num_symbols <= (c.pilot_symbols == 2 ? 11 : 2)) {
+    set_error("aft_synthetic_channels: bad grid %dx%d / pilots %dx%d (extents > 0, pilot_scs <= num_scs, pilot_symbols <= 2 at "
+              "symbols [2, 11] < num_symbols)", c.num_scs, c.num_symbols, c.pilot_scs, c.pilot_symbols);
+    return AFT_ERR_INVALID;
+  }
+  if (c.num_symbols > 256) {
+    set_error("aft_synthetic_channels: num_symbols %d not supported (<= 256)", c.num_symbols);
+    return AFT_ERR_UNSUPPORTED;
+  }
+  if (batch > 0 && (!snr || !delay_spread || !doppler || !pilots || !truth)) {
+    set_error("aft_synthetic_channels: NULL condition / pilots / truth buffer");
+    return AFT_ERR_INVALID;
+  }
+  if (batch > 0 && ((reinterpret_cast<uintptr_t>(pilots) | reinterpret_cast<uintptr_t>(truth)) & 7)) {
+    set_error("aft_synthetic_channels: pilots / truth not 8-byte aligned (complex64)");
+    return AFT_ERR_INVALID;
+  }
+  if (batch == 0) return AFT_OK;
+  return launch_synthetic_channels(c, seed, sample0, batch, snr, delay_spread, doppler, draw_conditions != 0,
+                                   static_cast<float2*>(pilots), static_cast<float2*>(truth), static_cast<cudaStream_t>(stream))
+             ? AFT_OK : AFT_ERR_CUDA;
+}
+
 int aft_profile_enable(AftHandle* h, int enable) {
   if (!h) { set_error("aft_profile_enable: NULL handle"); return AFT_ERR_INVALID; }
   h->profile = enable != 0;

@@ -136,6 +136,10 @@ size_t linear_backward_workspace_bytes(int64_t batch, int in_dim, int out_dim); 
 bool launch_linear_backward(const float* w, const float* x, const float* gy, float* grad_w, float* grad_b, float* grad_x,
                             int64_t batch, int in_dim, int out_dim, void* workspace, cudaStream_t st);
 
+// synth.cu : synthetic channels and noisy pilots (include/aft.h, "Synthetic channels"); arguments checked by the caller
+bool launch_synthetic_channels(const AftConfig& cfg, uint64_t seed, int64_t sample0, int64_t batch, float* snr, float* ds,
+                               float* dop, bool draw_conditions, float2* pilots, float2* truth, cudaStream_t st);
+
 // generic_f32.cu : AFT_FP32 path for non-default grids (activations in global memory, runtime extents)
 size_t generic_front_scratch_floats(int64_t nsamples, int P, int pix, int S);
 size_t generic_head_scratch_floats(int64_t nsamples, int pix);

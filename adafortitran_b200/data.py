@@ -6,10 +6,14 @@
   (``aft_extract_pilots``; device tensors in, device tensors out, ``ValueError`` on a wrong pilot count).
 * :class:`MatDataset` -- same ``__getitem__`` contract as the reference for ``.mat`` files holding ``H`` [scs, symbols, >=2];
   :func:`collate_on_device` stacks raw grids of a batch and extracts all pilots in one launch.
+* :class:`SyntheticChannels` -- training / evaluation batches generated on the GPU (``aft_synthetic_channels``) in the
+  form :func:`collate_on_device` returns; sample ``s`` of a seed is fixed by ``s`` alone, so data-parallel ranks generate
+  exactly their rows of the global batch.
 """
 from __future__ import annotations
 
 import ctypes as C
+import math
 import re
 from pathlib import Path
 from typing import Callable, List, Optional, Sequence, Tuple, Union
@@ -114,3 +118,73 @@ def collate_on_device(batch, pilot_size: Tuple[int, int], device: Union[str, tor
     truth = torch.stack([b[1] for b in batch]).to(device, non_blocking=True)
     meta = [torch.stack([b[2][k] for b in batch]) for k in range(5)] + [[tuple(b[2][5][0] for b in batch)]]
     return extract_pilots(grids, pilot_size), truth, tuple(meta)
+
+
+# The reference's condition grids (README.md:184-207): SNR dB, delay spread ns, maximum Doppler shift Hz.  The kernel draws
+# grid indices; these are the values it maps them to.
+SNR_GRID = tuple(float(v) for v in range(0, 31, 5))
+DS_GRID = tuple(float(v) for v in range(50, 351, 50))
+DOP_GRID = tuple(float(v) for v in range(200, 1401, 200))
+
+
+class SyntheticChannels:
+    """Doubly-selective channels and their noisy LS pilots, generated on the GPU (``include/aft.h``, "Synthetic
+    channels": 8 exponential-delay taps, Jakes-type Doppler, 15 kHz subcarriers, 14 symbols per ms, pilots at symbols
+    2 and 11).
+
+    ``system_config``: a :class:`SystemConfig` (or its dict) giving the grid and pilot extents.  ``seed``: 64-bit
+    integer naming the stream.  ``conditions``: ``None`` draws each sample's (SNR, delay spread, Doppler) from the
+    reference's 7 x 7 x 7 grid; ``(snr_db, delay_spread_ns, doppler_hz)`` fixes one condition for every sample.
+
+    :meth:`batch` ``(sample0, n)`` returns samples ``sample0 .. sample0 + n - 1`` of the stream as ``(pilots, meta,
+    truth)`` on the device, ``meta`` in the form of :func:`collate_on_device`, ready for ``model(pilots, meta)``,
+    ``ShardedTrainer.step`` and the evaluator.  A sample depends on the seed, its index and its condition only, so a
+    data-parallel rank calls ``batch(step * global_batch + lo, hi - lo)`` with its ``shard_range`` and gets exactly its
+    rows of ``batch(step * global_batch, global_batch)``."""
+
+    def __init__(self, system_config, seed: int, conditions: Optional[Tuple[float, float, float]] = None,
+                 device: Union[str, torch.device] = "cuda") -> None:
+        from .config import SystemConfig
+        if not isinstance(system_config, SystemConfig):
+            system_config = SystemConfig(**system_config)
+        self.system_config = system_config
+        seed = int(seed)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError(f"seed must be in [0, 2^64), got {seed}")
+        self.seed = seed
+        if conditions is not None:
+            snr, ds, dop = (float(v) for v in conditions)
+            if not all(math.isfinite(v) for v in (snr, ds, dop)) or ds <= 0 or dop < 0:
+                raise ValueError(f"conditions must be finite with delay spread > 0 and Doppler >= 0, got {conditions}")
+            conditions = (snr, ds, dop)
+        self.conditions = conditions
+        self.device = torch.device(device)
+        if self.device.type != "cuda":
+            raise RuntimeError("adafortitran_b200 has no CPU fallback: SyntheticChannels generates on a CUDA device")
+        o, p = system_config.ofdm, system_config.pilot
+        self._cfg = _capi.AftConfig(num_scs=o.num_scs, num_symbols=o.num_symbols, pilot_scs=p.num_scs,
+                                    pilot_symbols=p.num_symbols)
+
+    def batch(self, sample0: int, n: int):
+        """``(pilots c64 [n, pilot_scs, pilot_symbols], meta, truth c64 [n, num_scs, num_symbols])`` on the device.
+        ``meta`` = (sample index, snr, delay spread, Doppler, pilot spacing: five float32 ``[n, 1]`` tensors,
+        ``[("synthetic",) * n]``)."""
+        sample0, n = int(sample0), int(n)
+        o, p = self.system_config.ofdm, self.system_config.pilot
+        dev = self.device
+        pilots = torch.empty((n, p.num_scs, p.num_symbols), dtype=torch.complex64, device=dev)
+        truth = torch.empty((n, o.num_scs, o.num_symbols), dtype=torch.complex64, device=dev)
+        if self.conditions is None:
+            cond = torch.empty((3, n), dtype=torch.float32, device=dev)
+        else:
+            cond = torch.tensor(self.conditions, dtype=torch.float32, device=dev)[:, None].repeat(1, n)
+        ptr = lambda t: C.c_void_p(t.data_ptr()) if t.numel() else None
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            _capi.check(_capi.lib().aft_synthetic_channels(
+                C.byref(self._cfg), self.seed, sample0, n, ptr(cond[0]), ptr(cond[1]), ptr(cond[2]),
+                int(self.conditions is None), ptr(pilots), ptr(truth), C.c_void_p(stream)))
+        index = torch.arange(sample0, sample0 + n, dtype=torch.int64, device=dev).to(torch.float32)
+        spacing = torch.full((n,), float(o.num_scs // p.num_scs), dtype=torch.float32, device=dev)
+        meta = tuple(t.reshape(n, 1) for t in (index, cond[0], cond[1], cond[2], spacing)) + ([("synthetic",) * n],)
+        return pilots, meta, truth

@@ -212,6 +212,46 @@ AFT_API int aft_linear_backward(const float* weight, const float* x, const float
                                 float* grad_x, int64_t batch, int32_t in_dim, int32_t out_dim, void* workspace,
                                 size_t workspace_bytes, void* stream);
 
+/* ---- Synthetic channels ------------------------------------------------------------------------------------------
+ * Training and evaluation data generated on the device: a doubly-selective channel H (the truth) and its noisy pilots.
+ *
+ * Channel model, per sample: 8 taps t, each with a delay tau_t = -ds * 1e-9 * ln(u) seconds (ds = delay spread in ns),
+ * power p_t = exp(-tau_t / (ds * 1e-9)) / sum, i.e. u_t / sum_t' u_t', phase phi_t = 2 pi u and Doppler shift
+ * nu_t = f_d * cos(2 pi u) Hz (f_d = doppler).  With df = 15 kHz and Ts = 1e-3 / 14 s:
+ *   H[k, l] = sum_t sqrt(p_t) e^{j phi_t} e^{-j 2 pi k df tau_t} e^{j 2 pi nu_t l Ts}.
+ * Pilot i, m sits at subcarrier i * (num_scs / pilot_scs) (integer division) and symbol [2, 11][m]; its value is H there
+ * plus CN(0, sigma^2), sigma = 10^(-snr / 20), the two normals of each complex noise value from one Box-Muller pair.
+ *
+ * Random numbers: draw j of the sample with 64-bit global index s is Philox4x32-10 (the generator of the dropout masks)
+ * with key (seed & 0xffffffff, seed >> 32) and counter (j, s & 0xffffffff, s >> 32, 0x53594E54); the fourth word is never
+ * 0, so no draw equals a dropout draw.  Of an output word w, a uniform is u = ((w >> 8) | 1) * 2^-24, in (0, 1) and exact
+ * in fp32, and a grid index is ((w >> 8) * 7) >> 24, in 0..6.  The draws of a sample, in order:
+ *   j = 0          the condition (read only when drawn): snr = SNR[idx(w.x)], ds = DS[idx(w.y)], doppler = DOP[idx(w.z)]
+ *                  from the reference's grids SNR = 0, 5, .., 30 dB, DS = 50, 100, .., 350 ns, DOP = 200, 400, .., 1400 Hz;
+ *   j = 1 + t      tap t = 0..7: u(w.x) delay, u(w.y) phase, u(w.z) Doppler;
+ *   j = 9 + p / 2  the noise of pilot p = i * pilot_symbols + m: Box-Muller on (u(w.x), u(w.y)) for even p, on
+ *                  (u(w.z), u(w.w)) for odd p: (re, im) = sigma / sqrt(2) * sqrt(-2 ln u1) * (cos 2 pi u2, sin 2 pi u2).
+ * So a sample depends on (seed, s, its condition) only: any split of a batch into calls, chunks or ranks, each call with its
+ * sample0, gives the rows of one call over the whole batch bit for bit.
+ *
+ * Accuracy: k df tau_t reaches hundreds of turns; the delay and the turn counts are computed in fp64 and reduced to
+ * [-1/2, 1/2] before an fp32 sincospi, so H and the pilots are within ~1e-7 (normwise) of the model evaluated in fp64. */
+
+/* Generates samples sample0 .. sample0 + batch - 1 of the stream of `seed` for the grid and pilot extents of `cfg` (the
+ * other fields are ignored):
+ *   snr, delay_spread, doppler : float32 [batch] (device); with draw_conditions != 0 each sample's condition is drawn
+ *                                from the grids and written here, otherwise it is read from here
+ *   pilots : complex64 [batch, pilot_scs, pilot_symbols] (device, 8-byte aligned)
+ *   truth  : complex64 [batch, num_scs, num_symbols]     (device, 8-byte aligned; 16-byte stores when 16-byte aligned
+ *                                                         and num_symbols is even)
+ * Asynchronous on `stream`; no allocation, no host synchronisation.  AFT_ERR_INVALID with nothing launched for: NULL cfg;
+ * batch < 0, sample0 < 0 or sample0 + batch > INT64_MAX; a NULL or misaligned buffer with batch > 0; an extent <= 0,
+ * pilot_scs > num_scs, pilot_symbols > 2, or a pilot symbol index >= num_symbols.  AFT_ERR_UNSUPPORTED for num_symbols >
+ * 256.  batch == 0 launches nothing and returns AFT_OK. */
+AFT_API int aft_synthetic_channels(const AftConfig* cfg, uint64_t seed, int64_t sample0, int64_t batch, float* snr,
+                                   float* delay_spread, float* doppler, int32_t draw_conditions, void* pilots, void* truth,
+                                   void* stream);
+
 /* Number of kernel launches issued by this library on the calling process since load (for bench.py). */
 AFT_API int64_t aft_launch_count(void);
 
