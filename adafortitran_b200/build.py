@@ -26,11 +26,6 @@ NVCC_FLAGS = [
 ]
 
 
-def _extra_defs():
-    """Optional compile-time switches, e.g. AFT_NVCC_DEFS="-DAFT_TC_TIMELINE -DAFT_TC_PARTS=4" (diagnostics / experiments)."""
-    return [d for d in os.environ.get("AFT_NVCC_DEFS", "").split() if d]
-
-
 def _nvcc() -> str:
     for cand in (os.environ.get("NVCC"), shutil.which("nvcc"), "/usr/local/cuda/bin/nvcc"):
         if cand and os.path.exists(cand):
@@ -52,8 +47,10 @@ def _stale(target: str, deps) -> bool:
 VARIANTS = {
     # name -> extra nvcc defines.  "chaos": every mbarrier wait of the tensor-core kernels is preceded by a pseudo-random
     # delay (tc_ptx.cuh), which shakes the relative timing of the kernel's roles; used by the protocol test
-    # (tests/test_gpu_bf16.py::test_protocol_under_random_delays) through AFT_B200_LIB.
+    # (tests/test_gpu_bf16.py::test_protocol_under_random_delays) through AFT_B200_LIB.  "tl": the tensor-core kernels
+    # record in-kernel timelines (aft_selftest 102 / 103), read by tools/tc_check.py timeline and tools/conv_ab.sh.
     "chaos": ["-DAFT_TC_CHAOS"],
+    "tl": ["-DAFT_TC_TIMELINE"],
 }
 
 
@@ -63,42 +60,31 @@ def lib_file(variant: str | None = None) -> str:
 
 def build(force: bool = False, verbose: bool = False, variant: str | None = None) -> str:
     """Compile every ``csrc/*.cu`` for sm_100a and link ``libaft_b200.so`` (or a named variant).  Returns its path."""
-    global OBJ, LIB
-    if variant:
-        saved = (OBJ, LIB, os.environ.get("AFT_NVCC_DEFS"))
-        OBJ, LIB = os.path.join(PKG, f"build_{variant}"), lib_file(variant)
-        os.environ["AFT_NVCC_DEFS"] = " ".join(_extra_defs() + VARIANTS[variant])
-        try:
-            return build(force=force, verbose=verbose)
-        finally:
-            OBJ, LIB = saved[0], saved[1]
-            if saved[2] is None:
-                os.environ.pop("AFT_NVCC_DEFS", None)
-            else:
-                os.environ["AFT_NVCC_DEFS"] = saved[2]
-    os.makedirs(OBJ, exist_ok=True)
+    obj = os.path.join(PKG, f"build_{variant}") if variant else OBJ   # one object directory per variant
+    lib = lib_file(variant)
+    defs = VARIANTS[variant] if variant else []
+    os.makedirs(obj, exist_ok=True)
     os.makedirs(LIB_DIR, exist_ok=True)
     headers = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cuh", ".h"))]
     headers.append(os.path.join(os.path.dirname(PKG), "include", "aft.h"))
     nvcc = _nvcc()
-    stamp = os.path.join(OBJ, "defs.stamp")
-    defs = " ".join(_extra_defs())
-    if not os.path.exists(stamp) or open(stamp).read() != defs:
+    stamp = os.path.join(obj, "defs.stamp")
+    if not os.path.exists(stamp) or open(stamp).read() != " ".join(defs):
         force = True     # the compile-time switches changed: rebuild everything
         with open(stamp, "w") as f:
-            f.write(defs)
+            f.write(" ".join(defs))
     jobs = []
     for src in sources():
         s = os.path.join(CSRC, src)
-        o = os.path.join(OBJ, src[:-3] + ".o")
+        o = os.path.join(obj, src[:-3] + ".o")
         if force or _stale(o, [s] + headers):
             jobs.append((s, o))
 
     def compile_one(job):
         s, o = job
-        cmd = [nvcc] + NVCC_FLAGS + _extra_defs() + ["-c", s, "-o", o]
+        cmd = [nvcc] + NVCC_FLAGS + defs + ["-c", s, "-o", o]
         r = subprocess.run(cmd, capture_output=True, text=True)
-        log = os.path.join(OBJ, os.path.basename(s) + ".log")
+        log = os.path.join(obj, os.path.basename(s) + ".log")
         with open(log, "w") as f:
             f.write(" ".join(cmd) + "\n" + r.stdout + r.stderr)
         if r.returncode != 0:
@@ -110,19 +96,15 @@ def build(force: bool = False, verbose: bool = False, variant: str | None = None
     if jobs:
         with ThreadPoolExecutor(max_workers=min(8, len(jobs))) as ex:
             list(ex.map(compile_one, jobs))
-    objs = [os.path.join(OBJ, s[:-3] + ".o") for s in sources()]
-    if force or jobs or _stale(LIB, objs):
-        cmd = [nvcc, "-shared", "-o", LIB] + objs + ["-gencode", "arch=compute_100a,code=sm_100a", "-cudart", "static"]
+    objs = [os.path.join(obj, s[:-3] + ".o") for s in sources()]
+    if force or jobs or _stale(lib, objs):
+        cmd = [nvcc, "-shared", "-o", lib] + objs + ["-gencode", "arch=compute_100a,code=sm_100a", "-cudart", "static"]
         r = subprocess.run(cmd, capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError(f"link failed:\n{r.stdout}\n{r.stderr}")
-    return LIB
+    return lib
 
 
 if __name__ == "__main__":
     var = next((a.split("=", 1)[1] for a in sys.argv if a.startswith("--variant=")), None)
-    # ad-hoc experiment variant: --variant=NAME --defs="-DAFT_TC_TAILT=0 ..." builds lib/libaft_b200_NAME.so
-    extra = next((a.split("=", 1)[1] for a in sys.argv if a.startswith("--defs=")), None)
-    if var and extra is not None:
-        VARIANTS[var] = extra.split()
     print(build(force="--force" in sys.argv, verbose="-v" in sys.argv, variant=var))

@@ -13,10 +13,6 @@ using namespace convtc;
 
 namespace {
 
-#ifndef AFT_HEAD_L2_TC
-#define AFT_HEAD_L2_TC 1    // 1: linear_2 of the head as tcgen05 MMAs over the staged encoder image, 0: SIMT dot products
-#endif
-
 // One item = (token row t, 4 consecutive model columns): 288 x 32 items = 18 per thread.  A thread keeps the same four
 // columns for all its items (512 threads = 16 rows x 32 column groups per pass), so its IN_DIM x 4 weights stay in
 // registers as packed fp32 pairs and an item costs IN_DIM / 4 shared loads of the token row (one row per warp: broadcast)
@@ -243,10 +239,9 @@ head_tc_kernel(HeadPack p, const uint8_t* __restrict__ pack, const uint8_t* __re
 
   float* in = reinterpret_cast<float*>(smem + OFF_IN);
   const float* res = reinterpret_cast<const float*>(smem + OFF_OUT);
-  // persistent scratch (second a1 group): W2 image / weights 0..4095 | enhanced image 4096.. | real part 12288.. | complex64 staging row
+  // persistent scratch (second a1 group): W2 image 0..4095 | enhanced image 4096.. | real part 12288.. | complex64 staging row
   constexpr uint32_t kStageOff = OFF_KEEP + 19456;
   static_assert(12288 + kPix * 4 <= 19456 && 19456 + kPix * 8 <= kPlaneBytes, "staging row must fit behind the real part");
-#if AFT_HEAD_L2_TC
   // linear_2 on the tensor core.  The encoder's output image (2 K-chunks x 288 rows x 128 B, SWIZZLE_128B) is staged as ONE
   // contiguous 73,728-byte block starting 1024-aligned inside mid group 1 and running through groups 2 and 3 (dead between
   // two stack runs): it is then directly the A operand of  D[token, 16] = X[token, 128] . W2^T  (three M = 128 row tiles,
@@ -340,92 +335,6 @@ head_tc_kernel(HeadPack p, const uint8_t* __restrict__ pack, const uint8_t* __re
       }
       tc_fence_before_sync();
       __syncthreads();
-#else
-  // Input staging of one part: the encoder's output image (72 KB) goes into the position areas of mid groups 1..3 (dead
-  // between two stack runs; the guards between the groups stay zero), the enhanced image (fp32, 6.7 KB) behind the
-  // linear_2 weights in the persistent scratch.  Both arrive by bulk copies on the mbarrier at bar + 32.
-  auto img_addr = [&](uint32_t o) -> uint32_t { return sb + OFF_MID + (1 + (o >> 15)) * kPlaneBytes + kPosGuard * 16 + (o & 32767u); };
-  const float* es = reinterpret_cast<const float*>(smem + OFF_KEEP + 4096);
-  float* w2s = reinterpret_cast<float*>(smem + OFF_KEEP);   // linear_2 weights, [128][8] (k-major, 6 used), loaded once per CTA
-  float* re_keep = reinterpret_cast<float*>(smem + OFF_KEEP + 12288);   // real part of the sample (result of the first pass), [1680]
-  for (int i = tid; i < kD * 8; i += kThreads) {
-    const int k = i >> 3, f = i & 7;
-    w2s[i] = f < kPatchLen ? p.l2_w[f * kD + k] : 0.f;
-  }
-  __syncthreads();
-  uint32_t n_run = 0;
-
-  for (int64_t sample = blockIdx.x; sample < nsamples; sample += gridDim.x) {
-    for (int part = 0; part < 2; ++part, ++n_run) {
-      const int64_t seq = 2 * sample + part;
-      const uint8_t* hs = himg + seq * (int64_t)kXImageBytes;   // encoder output: bf16 operand image (tc_layout.cuh)
-#ifdef AFT_TC_TIMELINE
-      const bool st_on = blockIdx.x == 0 && n_run == 2 && tid == 0;
-      if (st_on) g_conv_tl[20] = clock64();
-#endif
-      if (tid == 0) {
-        // (the previous part ended with a __syncthreads: nobody reads the mid planes or the enhanced image any more)
-        mbar_arrive_expect_tx(bar + 32, kXImageBytes + kPix * sizeof(float));
-        bulk_g2s(img_addr(0), hs, 32768, bar + 32);
-        bulk_g2s(img_addr(32768), hs + 32768, 32768, bar + 32);
-        bulk_g2s(img_addr(65536), hs + 65536, kXImageBytes - 65536, bar + 32);
-        bulk_g2s(sb + OFF_KEEP + 4096, enh + seq * (int64_t)kPix, kPix * sizeof(float), bar + 32);
-        // the next part's inputs travel HBM -> L2 while this part's conv stack runs
-        const int64_t nseq2 = part == 0 ? seq + 1 : 2 * (sample + gridDim.x);
-        if (nseq2 < 2 * nsamples) {
-          bulk_prefetch_l2(himg + nseq2 * (int64_t)kXImageBytes, kXImageBytes);
-          bulk_prefetch_l2(enh + nseq2 * (int64_t)kPix, kPix * sizeof(float));
-        }
-      }
-      mbar_wait(bar + 32, n_run & 1);
-      // linear_2 (encoders.py:70), Fold (patch_processors.py:69-71) and the residual (fortitran.py:228).  Two threads per
-      // token, one per 64-column chunk of its image row; packed fp32x2 accumulation of the six outputs.
-      for (int base = 0; base < 2 * kS; base += kThreads) {
-        const int idx = base + tid;
-        const bool valid = idx < 2 * kS;           // whole warps run the shuffles below; only valid lanes store
-        const int t = valid ? idx >> 1 : 0, hf = idx & 1;
-        const uint32_t row = (uint32_t)(hf * kXChunkBytes + t * 128);
-        unsigned long long acc[3] = {0ull, 0ull, 0ull};            // (f0, f1), (f2, f3), (f4, f5) as packed fp32 pairs
-        const uint32_t wk = sb + OFF_KEEP + hf * 64 * 8 * 4;
-#pragma unroll
-        for (int u = 0; u < 8; ++u) {
-          uint4 v;
-          asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(img_addr(row + ((u ^ (t & 7)) << 4))));
-          const uint32_t w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-#pragma unroll
-            for (int e = 0; e < 2; ++e) {
-              const float x = e == 0 ? __uint_as_float(w[j] << 16) : __uint_as_float(w[j] & 0xFFFF0000u);
-              unsigned long long xx, w01, w23, w45;
-              asm("mov.b64 %0, {%1, %1};" : "=l"(xx) : "f"(x));
-              const uint32_t wa = wk + (u * 8 + 2 * j + e) * 32;
-              asm volatile("ld.shared.v2.b64 {%0, %1}, [%2];" : "=l"(w01), "=l"(w23) : "r"(wa));
-              asm volatile("ld.shared.b64 %0, [%1];" : "=l"(w45) : "r"(wa + 16));
-              asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc[0]) : "l"(xx), "l"(w01));
-              asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc[1]) : "l"(xx), "l"(w23));
-              asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc[2]) : "l"(xx), "l"(w45));
-            }
-          }
-        }
-        float a6[kPatchLen];
-#pragma unroll
-        for (int i = 0; i < 3; ++i) asm("mov.b64 {%0, %1}, %2;" : "=f"(a6[2 * i]), "=f"(a6[2 * i + 1]) : "l"(acc[i]));
-#pragma unroll
-        for (int f = 0; f < kPatchLen; ++f) a6[f] += __shfl_xor_sync(0xffffffffu, a6[f], 1);
-        // the pair shares the six outputs of the token: thread hf writes elements 3 hf .. 3 hf + 2 of the patch
-        const int pi = t / kTokW, pj = t - pi * kTokW;
-#pragma unroll
-        for (int ff = 0; ff < 3; ++ff) {
-          const int f = hf * 3 + ff;
-          const float val = hf ? a6[3 + ff] : a6[ff];
-          const int a = f / kPatchW, b = f - a * kPatchW;
-          const int r = kPatchH * pi + a, c = kPatchW * pj + b;
-          if (valid) in[(r + 1) * kPW + c + 1] = val + p.l2_b[f] + es[r * kGridW + c];
-        }
-      }
-      __syncthreads();
-#endif
 #ifdef AFT_TC_TIMELINE
       if (st_on) g_conv_tl[21] = clock64();
 #endif

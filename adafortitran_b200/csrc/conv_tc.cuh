@@ -37,10 +37,7 @@ constexpr int kPosGuard = 32;                 // positions of slack before p = 0
 constexpr int kPosAlloc = 2112;               // 32 guard + 2048 (16 M-tiles) + 32 guard
 constexpr int kPlaneBytes = kPosAlloc * 16;   // one 8-channel group: 33,792 bytes
 constexpr int kTiles = 16;
-#ifndef AFT_CONV_ISSUERS
-#define AFT_CONV_ISSUERS 4
-#endif
-constexpr int kIssuers = AFT_CONV_ISSUERS;       // warps that issue the MMAs of a conv layer (stack_run), = count of its mbarriers
+constexpr int kIssuers = 4;                   // warps that issue the MMAs of a conv layer (stack_run), = count of its mbarriers
 static_assert(kIssuers == 4, "a commit round (tiles 4 r .. 4 r + 3) must be the tiles one epilogue pass of the 16 warps reads");
 // mbarriers of a stack run, byte offsets from the `bar` block (OFF_BAR): one per round of four tiles and layer
 constexpr uint32_t kBarConv2 = 192, kBarConv3 = 224;

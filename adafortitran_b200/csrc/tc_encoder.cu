@@ -23,13 +23,13 @@
 //
 // GEMMs use M = 128 row tiles (3 per sequence; the rows past 280 of the third tile read whatever follows in shared
 // memory -- rows of A are independent, the corresponding accumulator lanes are never read); the attention of the
-// 24-row tail tile runs transposed (see "tail tile" below).
+// 24-row tail tile is sliced over the four lane quadrants (see "tail tile" below).
 //
 // Shared memory map (bytes, every region 1024-aligned; operand layouts in tc_layout.cuh):
 //   O    [      0,  73728)  attention output image (A of out_proj)   | FFN: hidden images, 2 x 36864
-//                           (padding rows 280..287: tail-tile exchange arrays, second mbarrier block)
+//                           (padding rows 280..287 of the second chunk: second mbarrier block)
 //   X    [  73728, 147456)  residual stream image (A of QKV / FFN1, residual of both LayerNorms)
-//   QKV  [ 147456, 202752)  Q_g | K_g | V_g of the current head, 288 x 64 B each (SWIZZLE_64B); P^T of the tail tile
+//   QKV  [ 147456, 202752)  Q_g | K_g | V_g of the current head, 288 x 64 B each (SWIZZLE_64B); P of the tail tile
 //                           | out_proj / FFN weight ring: 3 slots x 16384, then the layer's 4 KB vector block
 //   W    [ 202752, 227328)  in_proj slice of one head: rows q_g | k_g | v_g (96 x K=128) | FFN: second K-chunk of a W1 pair
 //   MISC [ 227328, 232448)  in_proj bias double buffer, mbarriers, TMEM base, softmax / LayerNorm exchange
@@ -53,33 +53,16 @@ namespace {
 using namespace ptx;
 using namespace tcm;
 
-#ifndef AFT_TC_POLY_EXP
-#define AFT_TC_POLY_EXP 3   // N > 0: in the full score tiles one pair of exponentials in N is evaluated on the FMA pipe (packed
-                            // fp32x2 Cody-Waite + cubic, 6 issue slots per value) instead of MUFU (8 pipe cycles per warp instruction)
-#endif
-#ifndef AFT_TC_PARTS
-#define AFT_TC_PARTS 4
-#endif
-#ifndef AFT_TC_GELU_TANH
-#define AFT_TC_GELU_TANH 1  // 1: GELU through one MUFU.TANH (erf-fitted odd polynomial argument), 0: erf by Abramowitz-Stegun (2 MUFU)
-#endif
-#ifndef AFT_TC_TAILT
-#define AFT_TC_TAILT 2      // tail tile (query rows 256..279) of every head -- 0: as a third row tile (one lane quadrant works),
-                            // 1: transposed (S^T, keys on the lanes), 2: sliced over the lane quadrants (see "tail tile, sliced")
-#endif
-#ifndef AFT_TC_SLICE2
-#define AFT_TC_SLICE2 0     // 1: the third row tile (rows 256..279) of the linear GEMMs is issued as N = 32 column slices, slice q with
-                            // its A operand starting 32 q rows earlier, so that quadrant q's lanes receive columns 32 q .. 32 q + 31 of
-                            // the tail rows and all four sub-partitions share that tile's epilogue (see "third row tile, sliced")
-#endif
-constexpr int kParts = AFT_TC_PARTS;   // threads per accumulator row = compute warpgroups (2: 8 warps x 224 regs, 4: 16 warps x 104 regs)
-static_assert(kParts == 2 || kParts == 4, "kParts must be 2 or 4");
+// In the score tiles one pair of exponentials in kPolyExp is evaluated on the FMA pipe (packed fp32x2 Cody-Waite + cubic,
+// 6 issue slots per value) instead of MUFU (8 pipe cycles per warp instruction), so that both pipes finish together.
+constexpr int kPolyExp = 3;
+constexpr int kParts = 4;   // threads per accumulator row = compute warpgroups (8 warps x 224 registers measured 7.6 % slower)
 static_assert(kXImageBytes % (16 * 32 * 4 * kParts) == 0, "the copy-out of the result image assumes whole passes of the compute warps");
 constexpr int kComputeWarps = 4 * kParts;
 constexpr int kTcThreads = 32 * (kComputeWarps + 4);   // compute warpgroups + [idle, idle, producer, MMA]
 constexpr int kProducerWarp = kComputeWarps + 2, kMmaWarp = kComputeWarps + 3;   // highest warp ids: favoured by the issue arbiter
 constexpr int kRegsCtrl = 56;                          // setmaxnreg budget of the control warpgroup
-constexpr int kRegsCompute = kParts == 2 ? 224 : 104;  // setmaxnreg budget of the compute warpgroups (pool = threads x launch regs)
+constexpr int kRegsCompute = 104;                      // setmaxnreg budget of the compute warpgroups (pool = threads x launch regs)
 // per-layer epilogue vectors (fp32, global): [4 heads][q32 | k32 | v32] in_proj bias (q part pre-scaled), then the
 // 1024-float block  b_out 128 | b_l1 256 | b_l2 128 | n1_w | n1_b | n2_w | n2_b  that is staged in shared memory
 constexpr int kVecPerLayer = 1408;
@@ -115,7 +98,7 @@ enum : uint32_t {
   MB_P_READY = 120,    // warp  : P tile written to TMEM
   MB_PV_DONE = 128,    // commit: P.V complete (P columns free, O accumulator valid)
   MB_O_FREE = 136,     // 2 x warp : O accumulator buffer b read out, O image columns written
-  MB_TAIL_MAX = 152,   // warp  : sliced tail, partial row maxima of every compute warp published
+  MB_TAIL_MAX = 152,   // warp  : tail tile, partial row maxima of every compute warp published
                        // (160, 224: free -- the per-tile OUT_DONE / X1_READY / X2_READY barriers live in the second block)
   MB_F1_DONE = 168,    // commit: FFN1 accumulator tile (128 rows x 128 hidden units) complete
   MB_F1_FREE = 176,    // warp  : FFN1 accumulator tile read out
@@ -134,34 +117,22 @@ constexpr uint32_t MISC_XSUM = MISC_XMAX + kXchgArray;   // exchange array 1 (so
 
 constexpr uint32_t TM_S = 0, TM_P = 288, TM_O = 432, TM_QKV = 0, TM_OUT = 0, TM_F1 = 384;
 // Accumulator columns of the QKV projection of (head g, row tile t).  Head 0 follows LayerNorm2 tile by tile and uses
-// columns t * 96 (inside the out_proj / FFN2 accumulators that LayerNorm2 has released up to that tile).  With the sliced
-// tail (AFT_TC_TAILT == 2) the tail scores of head g - 1 occupy all score columns, so for g > 0 tile 0 goes to the P
-// columns -- free as soon as P.V of the second score tile has completed: the tail's P lives in shared memory -- and is
-// issued BEFORE the tail's scores are read; tiles 1 and 2 follow in columns 0 and 96 while the tail's softmax runs.
+// columns t * 96 (inside the out_proj / FFN2 accumulators that LayerNorm2 has released up to that tile).  The tail
+// scores of head g - 1 occupy all score columns, so for g > 0 tile 0 goes to the P columns -- free as soon as P.V of the
+// second score tile has completed: the tail's P lives in shared memory -- and is issued BEFORE the tail's scores are
+// read; tiles 1 and 2 follow in columns 0 and 96 while the tail's softmax runs.
 __device__ __forceinline__ uint32_t qkv_col(int g, int t) {
-#if AFT_TC_TAILT == 2
   return g == 0 ? (uint32_t)(t * 96) : (t == 0 ? TM_P : (uint32_t)((t - 1) * 96));
-#else
-  (void)g;
-  return (uint32_t)(t * 96);
-#endif
 }
 
 constexpr uint32_t kIdescQkv = make_idesc_bf16(128, 96, false, false);
 constexpr uint32_t kIdescS = make_idesc_bf16(128, 144, false, false);
 constexpr uint32_t kIdescPV = make_idesc_bf16(128, 32, false, true);     // B = V, MN-major
 constexpr uint32_t kIdescN128 = make_idesc_bf16(128, 128, false, false);
-constexpr uint32_t kIdescST = make_idesc_bf16(128, 32, false, false);   // S^T block: A = 128 keys, B = 32 tail queries
-#ifndef AFT_TC_OT_M
-#define AFT_TC_OT_M 64
-#endif
-constexpr uint32_t kIdescOT = make_idesc_bf16(AFT_TC_OT_M, 32, true, true);
-constexpr uint32_t kIdescS96 = make_idesc_bf16(128, 96, false, false), kIdescS64 = make_idesc_bf16(128, 64, false, false);   // sliced tail: key slices
-constexpr uint32_t kIdescN32 = make_idesc_bf16(128, 32, false, false);   // column slices of the third row tile
-constexpr uint32_t kIdescPT = make_idesc_bf16(64, 32, false, true);    // sliced tail: O = P (image, K-major, M = 64) . V (MN-major)   // O^T: A = V^T (MN-major; only rows 0..31 = head dim matter), B = P^T (MN-major)
-// Tail tile exchange arrays ([4 quadrants][32 queries] f32 each): the padding rows 280..287 of the O image, chunk 0.
-// Those rows are never written during attention by the transposed path and out_proj only turns them into padding rows.
-constexpr uint32_t OFF_XT_MAX = OFF_O + 280 * 128, OFF_XT_SUM = OFF_XT_MAX + 512;
+constexpr uint32_t kIdescS96 = make_idesc_bf16(128, 96, false, false), kIdescS64 = make_idesc_bf16(128, 64, false, false);   // tail: key slices
+constexpr uint32_t kIdescPT = make_idesc_bf16(64, 32, false, true);    // tail: O = P (image, K-major, M = 64) . V (MN-major)
+// The padding rows 280..287 of the O image's first chunk are unused; those of its second chunk hold the second mbarrier
+// block (below).
 // Second LayerNorm exchange area (2 x kXchgArray bytes), used by row tile 1: the start of the O region.  Both LayerNorms run
 // when that region is dead (O image consumed by out_proj / hidden images consumed by FFN2, next writer behind a full
 // X1_READY / X2_READY hand-shake).
@@ -199,20 +170,6 @@ __device__ __forceinline__ void issue_gemm_sw128(uint32_t tmem, uint32_t d_col, 
     mma_ss(tmem + d_col, ((uint64_t)kHi << 32) | a, ((uint64_t)kHi << 32) | b, idesc, accumulate_first || ks > 0, el);
   }
 }
-// ---- third row tile, sliced (AFT_TC_SLICE2).  Only rows 256..279 of the third M = 128 row tile exist, and TMEM lane
-// quadrant q can only be read by the warps of sub-partition q: as one MMA the tile keeps a single sub-partition busy
-// through every epilogue (bias, LayerNorm, GELU) while the other three wait.  Row i of the A operand lands on lane i,
-// so the tile is issued as `nslices` N = 32 MMAs instead: slice q reads its A rows from 32 q rows EARLIER (tail rows on
-// the lanes of quadrant q; the rows in front are other tokens, their results are never read) and rows 32 q .. 32 q + 31
-// of B, and writes accumulator columns d_col + 32 q.  Quadrant q then owns output columns 32 q .. 32 q + 31 of the tail.
-// `a_row256` / `b_base`: shared addresses of row 256 of the A image and of row 0 of the B image (128-byte rows).
-__device__ __forceinline__ void issue_gemm_sw128_tail(uint32_t tmem, uint32_t d_col, uint32_t a_row256, uint32_t a_chunk_bytes,
-                                                      uint32_t b_base, uint32_t b_chunk_bytes, int ksteps, int nslices,
-                                                      bool accumulate_first, bool el = true) {
-  for (int qq = 0; qq < nslices; ++qq)
-    issue_gemm_sw128(tmem, d_col + 32 * qq, a_row256 - 4096 * qq, a_chunk_bytes, b_base + 4096 * qq, b_chunk_bytes, ksteps, kIdescN32,
-                     accumulate_first, el);
-}
 // Descriptors of the attention operands: constant high word (SBO | version | swizzle), low word = LBO | address >> 4,
 // so that stepping through an operand is one 32-bit add per MMA.
 constexpr uint32_t kDescHiSw64 = (uint32_t)(((uint64_t)(512 >> 4)) | ((uint64_t)1 << 14) | ((uint64_t)kSwizzle64 << 29));
@@ -237,32 +194,9 @@ __device__ __forceinline__ void issue_pv(uint32_t tmem, uint32_t sb, int obuf, b
   for (int ks = 0; ks < 18; ++ks) mma_ts(d, a + ks * 8, desc_sw64(v + ks * 64), kIdescPV, ks > 0, el);
 }
 
-// ---- tail tile (query rows 256..287), transposed.  TMEM lane quadrant w % 4 belongs to the warps of SM sub-partition
-// w % 4, so a 128 x 288 score tile with 32 valid rows keeps a single sub-partition (one MUFU) busy while 12 of the 16
-// compute warps wait.  Transposed, S^T = K_g . Q_tail^T puts the 288 keys on the lanes (three 128-lane blocks, N = 32
-// query columns each): every quadrant owns keys, the exponentials are spread over all four sub-partitions.  P^T is
-// written to shared memory with the layout of the V image (keys x 32, MN-major) over the dead Q image, and
-// O^T = V_g^T . P^T (A = V image read MN-major, lanes = head dim) lands in the usual O accumulator columns.
-__device__ __forceinline__ void issue_scores_tail(uint32_t tmem, uint32_t sb, bool el = true) {
-  const uint32_t k = desc_lo_k64(sb + OFF_QKV + kQkvPart);
-  const uint32_t qt = desc_lo_k64(sb + OFF_QKV + 256 * 64);
-#pragma unroll
-  for (int b = 0; b < 3; ++b)     // block 2 = keys 256..383: rows past 287 read the V image, their lanes are never loaded
-#pragma unroll
-    for (int ks = 0; ks < 2; ++ks)
-      mma_ss(tmem + TM_S + b * 32, desc_sw64(k + (b * 128 * 64) / 16 + ks * 2), desc_sw64(qt + ks * 2), kIdescST, ks > 0, el);
-}
-__device__ __forceinline__ void issue_pv_tail(uint32_t tmem, uint32_t sb, int obuf, bool el = true) {
-  const uint32_t v = desc_lo_mn64(sb + OFF_QKV + 2 * kQkvPart);
-  const uint32_t pt = desc_lo_mn64(sb + OFF_QKV);
-  const uint32_t d = tmem + TM_O + obuf * 32;
-  // A: M = 128 = four 32-wide MN atoms, only the first (lanes 0..31 = head dim) is meaningful; both strides of the
-  // descriptor are 512 B, so the other atoms read neighbouring key groups (in bounds, results ignored)
-#pragma unroll
-  for (int ks = 0; ks < 18; ++ks) mma_ss(d, desc_sw64(v + ks * 64), desc_sw64(pt + ks * 64), kIdescOT, ks > 0, el);
-}
-
-// ---- tail tile, sliced (AFT_TC_TAILT == 2).  Row i of an M = 128 A operand lands on TMEM lane i, and the A operand
+// ---- tail tile (query rows 256..279), sliced over the lane quadrants.  TMEM lane quadrant w % 4 belongs to the warps
+// of SM sub-partition w % 4, so a 128 x 288 score tile with 24 valid rows would keep a single sub-partition (one MUFU)
+// busy while 12 of the 16 compute warps wait.  Row i of an M = 128 A operand lands on TMEM lane i, and the A operand
 // is addressed by its first row: starting the Q image 32 q rows EARLIER puts the tail queries 256..279 on the lanes of
 // quadrant q (rows in front of them are other queries, their results are never read).  The tail scores are issued as
 // four such MMAs over disjoint key slices -- quadrant 0: keys [0, 96), quadrants 1..3: 64 keys each -- into the
@@ -271,7 +205,7 @@ __device__ __forceinline__ void issue_pv_tail(uint32_t tmem, uint32_t sb, int ob
 // the dead Q image (nine 32-key chunks of 32 rows x 64 B; an MMA reads past its chunk into the following ones: only
 // rows 0..23 matter), and O_tail = P . V runs as M = 64 MMAs into the usual accumulator columns.
 __device__ __forceinline__ int tail_key0(int q) { return q == 0 ? 0 : 32 + 64 * q; }   // 0, 96, 160, 224
-__device__ __forceinline__ void issue_scores_tail_sliced(uint32_t tmem, uint32_t sb, bool el = true) {
+__device__ __forceinline__ void issue_scores_tail(uint32_t tmem, uint32_t sb, bool el = true) {
 #pragma unroll
   for (int qq = 0; qq < 4; ++qq) {
     const int key0 = qq == 0 ? 0 : 32 + 64 * qq;
@@ -282,7 +216,7 @@ __device__ __forceinline__ void issue_scores_tail_sliced(uint32_t tmem, uint32_t
       mma_ss(tmem + TM_S + key0, desc_sw64(a + ks * 2), desc_sw64(k + ks * 2), qq == 0 ? kIdescS96 : kIdescS64, ks > 0, el);
   }
 }
-__device__ __forceinline__ void issue_pv_tail_sliced(uint32_t tmem, uint32_t sb, int obuf, bool el = true) {
+__device__ __forceinline__ void issue_pv_tail(uint32_t tmem, uint32_t sb, int obuf, bool el = true) {
   const uint32_t v = desc_lo_mn64(sb + OFF_QKV + 2 * kQkvPart);
   const uint32_t d = tmem + TM_O + obuf * 32;
 #pragma unroll
@@ -366,12 +300,11 @@ __device__ __forceinline__ float softmax_load(uint32_t tmem, int q, int part, fl
 // (2) exponentials in place (scores are in log2 units: q rows of in_proj pre-scaled by log2(e)/sqrt(dh)); returns the sum
 __device__ __forceinline__ float softmax_exp(float (&v)[kSmCols], float m) {
   float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-  // The exponentials are MUFU-bound (16 ex2 / clk / SM); every kPolyEvery-th one is computed on the FMA pipe instead
-  // so that both pipes finish together.
+  // The exponentials are MUFU-bound (16 ex2 / clk / SM); every fourth one is computed on the FMA pipe instead.
 #pragma unroll
   for (int j = 0; j < kSmCols; j += 4) {
     v[j] = ex2(v[j] - m); v[j + 1] = ex2(v[j + 1] - m); v[j + 2] = ex2(v[j + 2] - m);
-    v[j + 3] = AFT_TC_POLY_EXP ? ex2_poly(v[j + 3] - m) : ex2(v[j + 3] - m);
+    v[j + 3] = ex2_poly(v[j + 3] - m);
     s0 += v[j]; s1 += v[j + 1]; s2 += v[j + 2]; s3 += v[j + 3];
   }
   return (s0 + s1) + (s2 + s3);
@@ -383,12 +316,12 @@ __device__ __forceinline__ float softmax_exp_store(uint32_t tmem, int q, int par
   constexpr int kFull = kSmCols / 16;
   const f32x2 negm2 = pack2(-m, -m);
   f32x2 s2a = pack2(0.f, 0.f), s2b = pack2(0.f, 0.f);
-  // one pair of columns: subtract the row maximum, exponentiate (MUFU, or the FMA pipe for every AFT_TC_POLY_EXP-th pair),
+  // one pair of columns: subtract the row maximum, exponentiate (MUFU, or the FMA pipe for every kPolyExp-th pair),
   // accumulate the row sum, return the packed bf16 pair
   auto exp_pair = [&](int gp) -> uint32_t {
     const f32x2 x2 = add2(pack2(v[2 * gp], v[2 * gp + 1]), negm2);
     f32x2 e2;
-    if (AFT_TC_POLY_EXP > 0 && gp % (AFT_TC_POLY_EXP > 0 ? AFT_TC_POLY_EXP : 1) == (AFT_TC_POLY_EXP > 0 ? AFT_TC_POLY_EXP : 1) - 1) {
+    if (gp % kPolyExp == kPolyExp - 1) {
       e2 = ex2_poly2(x2);
     } else {
       float a, b;
@@ -461,157 +394,13 @@ __device__ __forceinline__ void epi_o_store(uint32_t sb, int g, int t, float inv
   epi_o_store_row(sb, g, t * 128 + q * 32 + lane, inv_l, part, a);
 }
 
-// ---- tail tile, transposed (see issue_scores_tail)
-constexpr int kTq = 32 / kParts;   // tail queries (accumulator columns per key block) per thread
-// Column-wise reduction over the 32 lanes of a warp: N values per lane in, and on return v[0] of lane L holds the
-// reduced column L >> (5 - log2 N) (N + log2(32 / N) - 1 shuffles instead of 5 N).
-template <int N, bool kMax>
-__device__ __forceinline__ void warp_reduce_cols(float (&v)[N], int lane, int width = 16) {
-  if constexpr (N > 1) {
-    const bool upper = (lane & width) != 0;
-    float h[N / 2];
-#pragma unroll
-    for (int i = 0; i < N / 2; ++i) {
-      const float send = upper ? v[i] : v[i + N / 2];
-      const float keep = upper ? v[i + N / 2] : v[i];
-      const float recv = __shfl_xor_sync(0xFFFFFFFFu, send, width);
-      h[i] = kMax ? fmaxf(keep, recv) : keep + recv;
-    }
-    warp_reduce_cols<N / 2, kMax>(h, lane, width >> 1);
-    v[0] = h[0];
-  } else {
-    for (; width >= 1; width >>= 1) {
-      const float recv = __shfl_xor_sync(0xFFFFFFFFu, v[0], width);
-      v[0] = kMax ? fmaxf(v[0], recv) : v[0] + recv;
-    }
-  }
-}
-__device__ __forceinline__ void st_shared_u16(uint32_t addr, uint32_t v) {
-  asm volatile("st.shared.u16 [%0], %1;" ::"r"(addr), "h"((unsigned short)v));
-}
-// Softmax of the transposed tail tile.  Thread (q, part, lane) owns keys 128 b + 32 q + lane (b = 0, 1 and, for q = 0,
-// b = 2) and tail queries part * kTq .. + kTq.  `s_loaded` / `part_bar`: see the call site.
-__device__ __forceinline__ void softmax_tail(uint32_t tmem, uint32_t sb, uint32_t s_loaded_bar, int q, int part, int lane) {
-  const int nb = q == 0 ? 3 : 2;
-  const uint32_t taddr = tmem + ((uint32_t)(q * 32) << 16) + TM_S + part * kTq;
-  float s[3][kTq];
-  {
-    uint32_t x[3][kTq];
-#pragma unroll
-    for (int b = 0; b < 3; ++b)
-      if (b < nb) tmem_ld_cols(taddr + b * 32, x[b]);
-    tmem_wait_ld();
-#pragma unroll
-    for (int b = 0; b < 3; ++b)
-#pragma unroll
-      for (int j = 0; j < kTq; ++j) s[b][j] = (b < nb) ? __uint_as_float(x[b][j]) : -INFINITY;
-  }
-  if (lane >= kS - 256) {   // keys 280..287 are padding
-#pragma unroll
-    for (int j = 0; j < kTq; ++j) s[2][j] = -INFINITY;
-  }
-  tc_fence_before_sync();
-  warp_arrive(s_loaded_bar, lane);
-  const int col_shift = kTq == 8 ? 2 : 1, col = lane >> col_shift;          // column held by this lane after a reduction
-  const bool writer = (lane & ((1 << col_shift) - 1)) == 0;
-  const uint32_t xslot = (q * 32 + part * kTq + col) * 4;
-  {
-    float m[kTq];
-#pragma unroll
-    for (int j = 0; j < kTq; ++j) m[j] = fmaxf(fmaxf(s[0][j], s[1][j]), s[2][j]);
-    warp_reduce_cols<kTq, true>(m, lane);
-    if (writer) st_shared_f32(sb + OFF_XT_MAX + xslot, m[0]);
-  }
-  named_bar_sync(5 + part, 128);   // the four quadrant warps that share these query columns
-  float sum[kTq];
-#pragma unroll
-  for (int u = 0; u < kTq / 4; ++u) {
-    float4 m4 = lds_f4(sb + OFF_XT_MAX + (part * kTq + u * 4) * 4);
-#pragma unroll
-    for (int qq = 1; qq < 4; ++qq) {
-      const float4 o = lds_f4(sb + OFF_XT_MAX + (qq * 32 + part * kTq + u * 4) * 4);
-      m4.x = fmaxf(m4.x, o.x); m4.y = fmaxf(m4.y, o.y); m4.z = fmaxf(m4.z, o.z); m4.w = fmaxf(m4.w, o.w);
-    }
-    // pairs of query columns; key block 1 goes through the FMA-pipe polynomial (one exponential in three, as in the
-    // full tiles), blocks 0 and 2 through the MUFU
-    const f32x2 nm[2] = {pack2(-m4.x, -m4.y), pack2(-m4.z, -m4.w)};
-#pragma unroll
-    for (int jp = 0; jp < 2; ++jp) {
-      const int j = u * 4 + 2 * jp;
-      f32x2 acc = pack2(0.f, 0.f);
-#pragma unroll
-      for (int b = 0; b < 3; ++b) {
-        if (b < nb) {
-          const f32x2 x2 = add2(pack2(s[b][j], s[b][j + 1]), nm[jp]);
-          f32x2 e2;
-          if (AFT_TC_POLY_EXP > 0 && b == 1) {
-            e2 = ex2_poly2(x2);
-          } else {
-            float a, c;
-            unpack2(x2, a, c);
-            e2 = pack2(ex2(a), ex2(c));
-          }
-          unpack2(e2, s[b][j], s[b][j + 1]);
-          acc = add2(acc, e2);
-        }
-      }
-      unpack2(acc, sum[j], sum[j + 1]);
-    }
-  }
-  // P^T rows (keys) -> the dead Q image, V-image layout: 64-byte rows, SWIZZLE_64B
-#pragma unroll
-  for (int b = 0; b < 3; ++b) {
-    if (b < nb) {
-      const int kr = b * 128 + q * 32 + lane;
-#pragma unroll
-      for (int u = 0; u < kTq / 8; ++u)
-        st_shared_v4(sb + OFF_QKV + kr * 64 + (((part * (kTq / 8) + u) ^ ((kr >> 1) & 3)) << 4),
-                     pack_bf16x2(s[b][8 * u], s[b][8 * u + 1]), pack_bf16x2(s[b][8 * u + 2], s[b][8 * u + 3]),
-                     pack_bf16x2(s[b][8 * u + 4], s[b][8 * u + 5]), pack_bf16x2(s[b][8 * u + 6], s[b][8 * u + 7]));
-    }
-  }
-  warp_reduce_cols<kTq, false>(sum, lane);
-  if (writer) st_shared_f32(sb + OFF_XT_SUM + xslot, sum[0]);
-}
-// O^T accumulator (lanes = head dim, columns = tail queries) -> / l -> bf16 -> O image rows 256..279 (quadrant 0 only)
-// With M = 64 the accumulator rows sit in 16-lane groups: row d lives in lane 32 (d / 16) + d % 16, i.e. head-dim rows
-// 0..15 in quadrant 0 and 16..31 in quadrant 1 (lanes 0..15 each); with M = 128 row d is lane d (quadrant 0 only).
-constexpr int kOtQuads = AFT_TC_OT_M == 64 ? 2 : 1;
-__device__ __forceinline__ void epi_o_tail(uint32_t tmem, uint32_t sb, int g, int obuf, int q, int part, int lane) {
-  uint32_t a[kTq];
-  tmem_ld_cols(tmem + ((uint32_t)(q * 32) << 16) + TM_O + obuf * 32 + part * kTq, a);
-  tmem_wait_ld();
-  if (AFT_TC_OT_M == 64 && lane >= 16) return;
-  const int d = AFT_TC_OT_M == 64 ? q * 16 + lane : lane;          // head-dim index of this thread's accumulator row
-  const uint32_t colbyte = (uint32_t)(d & 7) * 2;
-  const int u = (g & 1) * 4 + (d >> 3);
-#pragma unroll
-  for (int v4 = 0; v4 < kTq / 4; ++v4) {
-    float4 l4 = lds_f4(sb + OFF_XT_SUM + (part * kTq + v4 * 4) * 4);
-#pragma unroll
-    for (int qq = 1; qq < 4; ++qq) {
-      const float4 o = lds_f4(sb + OFF_XT_SUM + (qq * 32 + part * kTq + v4 * 4) * 4);
-      l4.x += o.x; l4.y += o.y; l4.z += o.z; l4.w += o.w;
-    }
-    const float ll[4] = {l4.x, l4.y, l4.z, l4.w};
-#pragma unroll
-    for (int jj = 0; jj < 4; ++jj) {
-      const int j = v4 * 4 + jj, r = 256 + part * kTq + j;
-      if (r < kS) {   // rows 280..287 hold the exchange arrays
-        const float o = __uint_as_float(a[j]) * rcp_approx(ll[jj]);
-        st_shared_u16(sb + OFF_O + (g >> 1) * kXChunkBytes + r * 128 + ((u ^ (r & 7)) << 4) + colbyte, pack_bf16x2(o, 0.f));
-      }
-    }
-  }
-}
-
-// ---- tail tile, sliced (see issue_scores_tail_sliced).  Thread (q, part, lane) owns tail query 256 + lane and NC keys:
+// ---- tail tile (see issue_scores_tail).  Thread (q, part, lane) owns tail query 256 + lane and NC keys:
 // tail_key0(q) + part * NC ...  The 16 threads of a row (4 quadrants x 4 warpgroups) exchange their partial maxima /
 // sums through the ordinary exchange arrays, each thread using the slot it also owns in the full tiles ([part][32 q +
 // lane]): a warp only overwrites slots of its own quadrant, whose previous readers (the quadrant's warps, second named
 // barrier of tile 1) are behind it, and the next full-tile writers are a whole QKV hand-shake away.
 template <int NC>
-__device__ __forceinline__ void softmax_tail_sliced_impl(uint32_t tmem, uint32_t sb, uint32_t miscb, uint32_t s_loaded_bar, uint32_t tail_bar, uint32_t tail_parity, int q, int part, int lane) {
+__device__ __forceinline__ void softmax_tail_impl(uint32_t tmem, uint32_t sb, uint32_t miscb, uint32_t s_loaded_bar, uint32_t tail_bar, uint32_t tail_parity, int q, int part, int lane) {
   static_assert(NC % 8 == 0, "a thread's keys must be whole 16-byte units of the P image");
   const int key0 = tail_key0(q) + part * NC;
   float v[NC];
@@ -651,7 +440,7 @@ __device__ __forceinline__ void softmax_tail_sliced_impl(uint32_t tmem, uint32_t
   for (int j = 0; j < NC / 2; ++j) {
     const f32x2 x2 = add2(pack2(v[2 * j], v[2 * j + 1]), negm2);
     f32x2 e2;
-    if (AFT_TC_POLY_EXP > 0 && j % 3 == 2) {
+    if (j % kPolyExp == kPolyExp - 1) {
       e2 = ex2_poly2(x2);
     } else {
       float a, b;
@@ -672,14 +461,14 @@ __device__ __forceinline__ void softmax_tail_sliced_impl(uint32_t tmem, uint32_t
   unpack2(s2, sa, sb2);
   st_shared_f32(miscb + MISC_XSUM + own, sa + sb2);
 }
-__device__ __forceinline__ void softmax_tail_sliced(uint32_t tmem, uint32_t sb, uint32_t miscb, uint32_t s_loaded_bar, uint32_t tail_bar,
-                                                    uint32_t tail_parity, int q, int part, int lane) {
-  static_assert(kParts == 4 || AFT_TC_TAILT != 2, "the sliced tail assumes four warpgroups");
-  if (q == 0) softmax_tail_sliced_impl<24>(tmem, sb, miscb, s_loaded_bar, tail_bar, tail_parity, q, part, lane);
-  else softmax_tail_sliced_impl<16>(tmem, sb, miscb, s_loaded_bar, tail_bar, tail_parity, q, part, lane);
+__device__ __forceinline__ void softmax_tail(uint32_t tmem, uint32_t sb, uint32_t miscb, uint32_t s_loaded_bar, uint32_t tail_bar,
+                                             uint32_t tail_parity, int q, int part, int lane) {
+  static_assert(kParts == 4, "the tail tile assumes four warpgroups");
+  if (q == 0) softmax_tail_impl<24>(tmem, sb, miscb, s_loaded_bar, tail_bar, tail_parity, q, part, lane);
+  else softmax_tail_impl<16>(tmem, sb, miscb, s_loaded_bar, tail_bar, tail_parity, q, part, lane);
 }
 // O_tail accumulator (M = 64: tail query i in lane i % 16 of quadrant i / 16) -> / l -> bf16 -> O image rows 256..279
-__device__ __forceinline__ void epi_o_tail_sliced(uint32_t tmem, uint32_t sb, uint32_t miscb, int g, int obuf, int q, int part, int lane) {
+__device__ __forceinline__ void epi_o_tail(uint32_t tmem, uint32_t sb, uint32_t miscb, int g, int obuf, int q, int part, int lane) {
   uint32_t a[kOCols];
   tmem_ld_cols(tmem + ((uint32_t)(q * 32) << 16) + TM_O + obuf * 32 + part * kOCols, a);
   tmem_wait_ld();
@@ -760,8 +549,8 @@ __device__ __forceinline__ void epi_ln(uint32_t tmem, uint32_t sb, uint32_t vec,
     f32x2 o[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) o[j] = fma2(fma2(v[u * 4 + j], rstd2, shift2), gg[j], ee[j]);
-    // padding rows 280..287 stay zero: their accumulators are fed by padding rows of the O image (exchange scratch of
-    // the tail tile) and must not leak non-finite values into the V image of the next layer
+    // padding rows 280..287 stay zero: their accumulators are fed by padding rows of the O region (which hold the second
+    // mbarrier block) and must not leak non-finite values into the V image of the next layer
     if (r < kS) {
       const uint4 pk = make_uint4(pack_bf16_pair(o[0]), pack_bf16_pair(o[1]), pack_bf16_pair(o[2]), pack_bf16_pair(o[3]));
       const uint32_t off = r * 128 + (((u0 + u) ^ (r & 7)) << 4);
@@ -772,113 +561,6 @@ __device__ __forceinline__ void epi_ln(uint32_t tmem, uint32_t sb, uint32_t vec,
   }
   // No trailing barrier: consecutive tiles alternate between two exchange areas (see the call sites), and a warp can only
   // reach tile t + 2 after every warp of its quadrant has passed the barrier of tile t + 1, i.e. finished reading tile t.
-}
-
-// ---- third row tile, sliced: epilogues.  Thread (q, part, lane) owns row 256 + lane and the 8 output columns
-// c0 = 32 q + 8 part ... of it (QKV: quadrant q < 3 holds matrix q of [q | k | v], columns 8 part ...).
-constexpr int kSliceBar = 12;   // named barrier of all compute warps: LayerNorm partial sums of the third row tile exchanged
-__device__ __forceinline__ void epi_qkv_tail(uint32_t tmem, uint32_t sb, uint32_t bias96, int g, int q, int part, int lane) {
-  uint32_t a[8];
-  tmem_ld_cols(tmem + ((uint32_t)(q * 32) << 16) + qkv_col(g, 2) + q * 32 + part * 8, a);
-  const uint4 b0 = ld_shared_v4(bias96 + (q * 32 + part * 8) * 4), b1 = ld_shared_v4(bias96 + (q * 32 + part * 8) * 4 + 16);
-  tmem_wait_ld();
-  const int r = 256 + lane;
-  auto sum = [](uint32_t x0, uint32_t x1, uint32_t y0, uint32_t y1) {
-    return pack_bf16_pair(add2(pack2(__uint_as_float(x0), __uint_as_float(x1)), pack2(__uint_as_float(y0), __uint_as_float(y1))));
-  };
-  st_shared_v4(sb + OFF_QKV + q * kQkvPart + r * 64 + ((part ^ ((r >> 1) & 3)) << 4), sum(a[0], a[1], b0.x, b0.y), sum(a[2], a[3], b0.z, b0.w),
-               sum(a[4], a[5], b1.x, b1.y), sum(a[6], a[7], b1.z, b1.w));
-}
-// out_proj / linear2 + bias + residual -> LayerNorm -> X rows 256..279.  The 16 threads of a row exchange their partial
-// sums through `xchg` (two kXchgArray areas), each in the slot it owns in the full tiles ([part][32 q + lane]).
-__device__ __forceinline__ void epi_ln_tail(uint32_t tmem, uint32_t sb, uint32_t vec, int which, int q, int part, int lane, uint32_t xchg) {
-  const int r = 256 + lane, c0 = q * 32 + part * 8;
-  const uint32_t bias = vec + 4 * ((which == 1 ? kVecBOut : kVecBL2) + c0);
-  const uint32_t gam = vec + 4 * ((which == 1 ? kVecN1W : kVecN2W) + c0);
-  const uint32_t bet = vec + 4 * ((which == 1 ? kVecN1B : kVecN2B) + c0);
-  const uint32_t xaddr = sb + OFF_X + (c0 >> 6) * kXChunkBytes + r * 128 + (((((c0 & 63) >> 3)) ^ (r & 7)) << 4);
-  uint32_t acc[8];
-  tmem_ld_cols(tmem + ((uint32_t)(q * 32) << 16) + TM_OUT + 256 + c0, acc);
-  const uint4 xr = ld_shared_v4(xaddr);
-  const uint4 b0 = ld_shared_v4(bias), b1 = ld_shared_v4(bias + 16);
-  tmem_wait_ld();
-  const uint32_t xw[4] = {xr.x, xr.y, xr.z, xr.w};
-  const f32x2 bb[4] = {pack2(__uint_as_float(b0.x), __uint_as_float(b0.y)), pack2(__uint_as_float(b0.z), __uint_as_float(b0.w)),
-                       pack2(__uint_as_float(b1.x), __uint_as_float(b1.y)), pack2(__uint_as_float(b1.z), __uint_as_float(b1.w))};
-  f32x2 v[4], s2 = pack2(0.f, 0.f), q2 = pack2(0.f, 0.f);
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    const f32x2 a2 = pack2(__uint_as_float(acc[2 * j]), __uint_as_float(acc[2 * j + 1]));
-    v[j] = add2(add2(a2, bb[j]), bf16x2_to_f32x2(xw[j]));
-    s2 = add2(s2, v[j]);
-    q2 = fma2(v[j], v[j], q2);
-  }
-  {
-    float sa, sb2, qa, qb;
-    unpack2(s2, sa, sb2);
-    unpack2(q2, qa, qb);
-    st_shared_f32(xchg + (part * 128 + q * 32 + lane) * 4, sa + sb2);
-    st_shared_f32(xchg + kXchgArray + (part * 128 + q * 32 + lane) * 4, qa + qb);
-  }
-  named_bar_sync(kSliceBar, 32 * kComputeWarps);
-  float sum = 0.f, sq = 0.f;
-#pragma unroll
-  for (int pp = 0; pp < 4; ++pp)
-#pragma unroll
-    for (int qq = 0; qq < 4; ++qq) {
-      sum += ld_shared_f32(xchg + (pp * 128 + qq * 32 + lane) * 4);
-      sq += ld_shared_f32(xchg + kXchgArray + (pp * 128 + qq * 32 + lane) * 4);
-    }
-  const float mean = sum * (1.0f / 128.0f);
-  const float var = fmaxf(fmaf(-mean, mean, sq * (1.0f / 128.0f)), 0.f);
-  const float rstd = rsqrtf(var + 1e-5f);
-  const float shift = -mean * rstd;
-  const f32x2 rstd2 = pack2(rstd, rstd), shift2 = pack2(shift, shift);
-  const uint4 g0 = ld_shared_v4(gam), g1 = ld_shared_v4(gam + 16), e0 = ld_shared_v4(bet), e1 = ld_shared_v4(bet + 16);
-  const f32x2 gg[4] = {pack2(__uint_as_float(g0.x), __uint_as_float(g0.y)), pack2(__uint_as_float(g0.z), __uint_as_float(g0.w)),
-                       pack2(__uint_as_float(g1.x), __uint_as_float(g1.y)), pack2(__uint_as_float(g1.z), __uint_as_float(g1.w))};
-  const f32x2 ee[4] = {pack2(__uint_as_float(e0.x), __uint_as_float(e0.y)), pack2(__uint_as_float(e0.z), __uint_as_float(e0.w)),
-                       pack2(__uint_as_float(e1.x), __uint_as_float(e1.y)), pack2(__uint_as_float(e1.z), __uint_as_float(e1.w))};
-  if (r < kS) {   // padding rows 280..287 stay zero
-    f32x2 o[4];
-#pragma unroll
-    for (int j = 0; j < 4; ++j) o[j] = fma2(fma2(v[j], rstd2, shift2), gg[j], ee[j]);
-    st_shared_v4(xaddr, pack_bf16_pair(o[0]), pack_bf16_pair(o[1]), pack_bf16_pair(o[2]), pack_bf16_pair(o[3]));
-  }
-}
-// FFN1 accumulators of the third row tile: load + bias, then GELU / ReLU -> hidden image rows 256..279
-__device__ __forceinline__ void act_tail_load(uint32_t tmem, uint32_t vec, int pr, int q, int part, f32x2 (&f)[4]) {
-  const int c0 = q * 32 + part * 8;
-  const uint32_t bias = vec + 4 * (kVecBL1 + pr * 128 + c0);
-  uint32_t a[8];
-  tmem_ld_cols(tmem + ((uint32_t)(q * 32) << 16) + TM_F1 + c0, a);
-  const uint4 b0 = ld_shared_v4(bias), b1 = ld_shared_v4(bias + 16);
-  tmem_wait_ld();
-  f[0] = add2(pack2(__uint_as_float(a[0]), __uint_as_float(a[1])), pack2(__uint_as_float(b0.x), __uint_as_float(b0.y)));
-  f[1] = add2(pack2(__uint_as_float(a[2]), __uint_as_float(a[3])), pack2(__uint_as_float(b0.z), __uint_as_float(b0.w)));
-  f[2] = add2(pack2(__uint_as_float(a[4]), __uint_as_float(a[5])), pack2(__uint_as_float(b1.x), __uint_as_float(b1.y)));
-  f[3] = add2(pack2(__uint_as_float(a[6]), __uint_as_float(a[7])), pack2(__uint_as_float(b1.z), __uint_as_float(b1.w)));
-}
-__device__ __forceinline__ void act_tail_store(uint32_t sb, int act, int q, int part, int lane, f32x2 (&f)[4]) {
-  const int r = 256 + lane, c0 = q * 32 + part * 8;
-  uint32_t pk[4];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    if (act == AFT_ACT_GELU) {
-      if (AFT_TC_GELU_TANH) {
-        pk[j] = pack_bf16_pair(gelu_tanh2(f[j]));
-      } else {
-        float a, b;
-        unpack2(f[j], a, b);
-        pk[j] = pack_bf16x2(gelu_fast(a), gelu_fast(b));
-      }
-    } else {
-      float a, b;
-      unpack2(f[j], a, b);
-      pk[j] = pack_bf16x2(fmaxf(a, 0.f), fmaxf(b, 0.f));
-    }
-  }
-  if (r < kS) st_shared_v4(sb + OFF_O + (c0 >> 6) * kHidBytes + r * 128 + (((((c0 & 63) >> 3)) ^ (r & 7)) << 4), pk[0], pk[1], pk[2], pk[3]);
 }
 
 // FFN1 accumulators (pair pr = hidden units 128 pr .. 128 pr + 127, one row tile), split over the warpgroups: load + bias
@@ -902,15 +584,7 @@ __device__ __forceinline__ void act_store(uint32_t sb, int t, int act, int q, in
   uint32_t pk[kActCols / 2];
   if (act == AFT_ACT_GELU) {
 #pragma unroll
-    for (int j = 0; j < kActCols / 2; ++j) {
-      if (AFT_TC_GELU_TANH) {
-        pk[j] = pack_bf16_pair(gelu_tanh2(f[j]));
-      } else {
-        float a, b;
-        unpack2(f[j], a, b);
-        pk[j] = pack_bf16x2(gelu_fast(a), gelu_fast(b));
-      }
-    }
+    for (int j = 0; j < kActCols / 2; ++j) pk[j] = pack_bf16_pair(gelu_tanh2(f[j]));
   } else {
 #pragma unroll
     for (int j = 0; j < kActCols / 2; ++j) {
@@ -1084,12 +758,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) encoder_kernel(EncParams p) {
               tc_fence_after_sync();
               tl_event(p, tl, 100 + g, tl_n);   // QKV(g) issue start
             }
-            for (int t = t0; t < t1; ++t) {
-              if (AFT_TC_SLICE2 && t == 2)   // third row tile: one N = 32 slice per matrix (q | k | v) on quadrants 0..2
-                issue_gemm_sw128_tail(tmem, qkv_col(g, 2), sb + OFF_X + 256 * 128, kXChunkBytes, sb + OFF_W, 96 * 128, 8, 3, false, el);
-              else
-                issue_gemm_sw128(tmem, qkv_col(g, t), sb + OFF_X + t * 128 * 128, kXChunkBytes, sb + OFF_W, 96 * 128, 8, kIdescQkv, false, el);
-            }
+            for (int t = t0; t < t1; ++t)
+              issue_gemm_sw128(tmem, qkv_col(g, t), sb + OFF_X + t * 128 * 128, kXChunkBytes, sb + OFF_W, 96 * 128, 8, kIdescQkv, false, el);
             if (last) {
               mma_commit(misc + MB_W_EMPTY, el);
               mma_commit(misc + MB_QKV_DONE, el);
@@ -1123,43 +793,20 @@ __global__ void __launch_bounds__(kTcThreads, 1) encoder_kernel(EncParams p) {
               s_loaded.wait(misc + MB_S_LOADED);      // S(t) is in registers
               tc_fence_after_sync();
               tl_event(p, tl, 130 + t, tl_n);   // S_LOADED(t) seen
-#if AFT_TC_TAILT == 2
               if (t == 0) { issue_scores(tmem, sb, 1, el); mma_commit(misc + MB_S_DONE, el); }
-              else if (t == 1) { issue_scores_tail_sliced(tmem, sb, el); mma_commit(misc + MB_S_DONE, el); }
-              // the sliced tail scores fill all score columns: row tiles 1 and 2 of the next head's projection follow their
+              else if (t == 1) { issue_scores_tail(tmem, sb, el); mma_commit(misc + MB_S_DONE, el); }
+              // the tail scores fill all score columns: row tiles 1 and 2 of the next head's projection follow their
               // read-out and run under the tail's softmax (tile 0 was issued into the P columns, see below).  Measured:
               // holding tile 2 back until P.V of the tail has been issued is slower (57.5 vs 56.6 ms per 16384 estimates).
               else if (g < 3) issue_qkv(g + 1, 1, 3, false, true);
-#elif AFT_TC_TAILT
-              if (t == 0) { issue_scores(tmem, sb, 1, el); mma_commit(misc + MB_S_DONE, el); }
-              else if (t == 1) {
-                issue_scores_tail(tmem, sb, el);
-                mma_commit(misc + MB_S_DONE, el);
-                // S^T only occupies columns [0, 96): row tiles 1 and 2 of the next head's projection start right away
-                if (g < 3) issue_qkv(g + 1, 1, 3, true, false);
-              }
-              else if (g < 3) issue_qkv(g + 1, 0, 1, false, true);
-#else
-              // the S columns are free after the last tile: the next head's projection runs under this tile's exponentials
-              // (it only reads X and the weight slot; the Q/K/V images are rewritten later, by the epilogue)
-              if (t < 2) { issue_scores(tmem, sb, t + 1, el); mma_commit(misc + MB_S_DONE, el); }
-              else if (g < 3) issue_qkv(g + 1, 0, 3, true, true);
-#endif
               p_ready.wait(misc + MB_P_READY);         // P(t) is in TMEM
               // O accumulator n_pv & 1 was last used by P.V #(n_pv - 2): its epilogue must have read it out
               if (n_pv >= 2) mbar_wait(misc + MB_O_FREE + 8 * (n_pv & 1), ((n_pv >> 1) - 1) & 1);
               tc_fence_after_sync();
               tl_event(p, tl, 140 + t, tl_n);   // P_READY(t) seen, P.V(t) issue start
-#if AFT_TC_TAILT == 2
-              if (t == 2) issue_pv_tail_sliced(tmem, sb, n_pv & 1, el); else issue_pv(tmem, sb, n_pv & 1, el);
-#elif AFT_TC_TAILT
               if (t == 2) issue_pv_tail(tmem, sb, n_pv & 1, el); else issue_pv(tmem, sb, n_pv & 1, el);
-#else
-              issue_pv(tmem, sb, n_pv & 1, el);
-#endif
               mma_commit(misc + MB_PV_DONE, el);
               tl_event(p, tl, 150 + t, tl_n);   // P.V(t) issued
-#if AFT_TC_TAILT == 2
               if (t == 1 && g < 3) {
                 // row tile 0 of the next head's projection -> P columns: P.V(1) (the last reader of P in TMEM for this head)
                 // must have completed; nothing else is pending for this warp until the tail's scores have been read
@@ -1167,7 +814,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) encoder_kernel(EncParams p) {
                 tc_fence_after_sync();
                 issue_qkv(g + 1, 0, 1, true, false);
               }
-#endif
               if (g == 3 && t == 2) mma_commit(misc + MB_ATTN_DONE, el);
             }
           }
@@ -1180,13 +826,8 @@ __global__ void __launch_bounds__(kTcThreads, 1) encoder_kernel(EncParams p) {
             tl_event(p, tl, 160, tl_n);   // out_proj issue start
             const uint32_t w0 = ring_wait(ring_base + 0), w1 = ring_wait(ring_base + 1);
             for (int t = 0; t < 3; ++t) {   // tile-major: LayerNorm1 of tile 0 starts while tiles 1 and 2 are still in the pipe
-              if (AFT_TC_SLICE2 && t == 2) {
-                issue_gemm_sw128_tail(tmem, TM_OUT + 256, sb + OFF_O + 256 * 128, 0, w0, 0, 4, 4, false, el);
-                issue_gemm_sw128_tail(tmem, TM_OUT + 256, sb + OFF_O + kXChunkBytes + 256 * 128, 0, w1, 0, 4, 4, true, el);
-              } else {
-                issue_gemm_sw128(tmem, TM_OUT + t * 128, sb + OFF_O + t * 128 * 128, 0, w0, 0, 4, kIdescN128, false, el);
-                issue_gemm_sw128(tmem, TM_OUT + t * 128, sb + OFF_O + kXChunkBytes + t * 128 * 128, 0, w1, 0, 4, kIdescN128, true, el);
-              }
+              issue_gemm_sw128(tmem, TM_OUT + t * 128, sb + OFF_O + t * 128 * 128, 0, w0, 0, 4, kIdescN128, false, el);
+              issue_gemm_sw128(tmem, TM_OUT + t * 128, sb + OFF_O + kXChunkBytes + t * 128 * 128, 0, w1, 0, 4, kIdescN128, true, el);
               mma_commit(bar2 + MB2_OUT_DONE + 8 * t, el);
             }
             ring_release(ring_base + 0);
@@ -1207,10 +848,6 @@ __global__ void __launch_bounds__(kTcThreads, 1) encoder_kernel(EncParams p) {
               tc_fence_after_sync();
               const uint32_t w2a = ring_wait(ring_base + 3 + 3 * pj), w2b = ring_wait(ring_base + 4 + 3 * pj);
               const uint32_t d = tmem + TM_OUT + tj * 128;
-              if (AFT_TC_SLICE2 && tj == 2) {
-                issue_gemm_sw128_tail(tmem, TM_OUT + 256, sb + OFF_O + 256 * 128, 0, w2a, 0, 4, 4, pj > 0, el);
-                issue_gemm_sw128_tail(tmem, TM_OUT + 256, sb + OFF_O + kHidBytes + 256 * 128, 0, w2b, 0, 4, 4, true, el);
-              } else
 #pragma unroll
               for (int cc = 0; cc < 2; ++cc) {
                 const uint32_t a_lo = desc128(sb + OFF_O + cc * kHidBytes + tj * 128 * 128), b_lo = desc128(cc == 0 ? w2a : w2b);
@@ -1235,17 +872,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) encoder_kernel(EncParams p) {
               if (pr == 0) mbar_wait(bar2 + MB2_X1_READY + 8 * t, n_layers_done & 1);   // LayerNorm1 rows of this tile are in X
               if (n_f1 >= 1) mbar_wait(misc + MB_F1_FREE, (n_f1 - 1) & 1);
               tc_fence_after_sync();
-              if (AFT_TC_SLICE2 && t == 2) {
-                issue_gemm_sw128_tail(tmem, TM_F1, sb + OFF_X + 256 * 128, 0, w1a, 0, 4, 4, false, el);
-                issue_gemm_sw128_tail(tmem, TM_F1, sb + OFF_X + kXChunkBytes + 256 * 128, 0, w1b, 0, 4, 4, true, el);
-              } else {
-                const uint32_t a0 = desc128(sb + OFF_X + t * 128 * 128), a1 = desc128(sb + OFF_X + kXChunkBytes + t * 128 * 128);
-                const uint32_t b0 = desc128(w1a), b1 = desc128(w1b);
+              const uint32_t a0 = desc128(sb + OFF_X + t * 128 * 128), a1 = desc128(sb + OFF_X + kXChunkBytes + t * 128 * 128);
+              const uint32_t b0 = desc128(w1a), b1 = desc128(w1b);
 #pragma unroll
-                for (int ks = 0; ks < 8; ++ks)
-                  mma_ss(tmem + TM_F1, ((uint64_t)kHi << 32) | ((ks < 4 ? a0 : a1) + (ks & 3) * 2),
-                         ((uint64_t)kHi << 32) | ((ks < 4 ? b0 : b1) + (ks & 3) * 2), kIdescN128, ks > 0, el);
-              }
+              for (int ks = 0; ks < 8; ++ks)
+                mma_ss(tmem + TM_F1, ((uint64_t)kHi << 32) | ((ks < 4 ? a0 : a1) + (ks & 3) * 2),
+                       ((uint64_t)kHi << 32) | ((ks < 4 ? b0 : b1) + (ks & 3) * 2), kIdescN128, ks > 0, el);
               mma_commit(misc + MB_F1_DONE, el);
               tl_event(p, tl, 180 + k, tl_n);   // FFN1(k) issued
               if (t == 2) {   // the pair's weights are free once these MMAs have completed
@@ -1290,17 +922,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) encoder_kernel(EncParams p) {
           tc_fence_after_sync();
           tl_event(p, tl, 210 + g, tl_n);   // QKV_DONE seen
           epi_qkv_pair(tmem, sb, qb, g, q, part, lane);
-#if AFT_TC_SLICE2
-          if (q < 3) epi_qkv_tail(tmem, sb, qkv_bias + (g & 1) * kQkvBiasBytes, g, q, part, lane);
-#else
           if (tile2_active) epi_qkv(tmem, sb, qb, g, 2, q, part, lane);
-#endif
           tc_fence_before_sync();
           fence_proxy_async_smem();
           warp_arrive(misc + MB_QKV_READY, lane);
           tl_event(p, tl, 220 + g, tl_n);   // QKV epilogue done
           // ---- softmax tiles; the O epilogue of tile t-1 runs after P(t) has been handed to the tensor core
-#if AFT_TC_TAILT
           float inv_prev = 0.f;
 #pragma unroll 1
           for (int t = 0; t < 4; ++t) {
@@ -1340,30 +967,22 @@ __global__ void __launch_bounds__(kTcThreads, 1) encoder_kernel(EncParams p) {
             } else if (t == 2) {
               mbar_wait(misc + MB_S_DONE, (n_head + 2) & 1);
               tc_fence_after_sync();
-              tl_event(p, tl, 232, tl_n);       // S^T seen
-#if AFT_TC_TAILT == 2
-              softmax_tail_sliced(tmem, sb, miscb, misc + MB_S_LOADED, misc + MB_TAIL_MAX, n_head & 1, q, part, lane);
-#else
-              softmax_tail(tmem, sb, misc + MB_S_LOADED, q, part, lane);
-#endif
-              fence_proxy_async_smem();         // P^T / P is read by the tensor core
+              tl_event(p, tl, 232, tl_n);       // tail S seen
+              softmax_tail(tmem, sb, miscb, misc + MB_S_LOADED, misc + MB_TAIL_MAX, n_head & 1, q, part, lane);
+              fence_proxy_async_smem();         // P is read by the tensor core
               // P.V(1) (long finished): waited for before the arrival so that the PV_DONE barrier can never run two
               // phases ahead of a waiter; its O accumulator is read out right below
               mbar_wait(misc + MB_PV_DONE, (n_head + 1) & 1);
               tc_fence_after_sync();
               warp_arrive(misc + MB_P_READY, lane);
-              tl_event(p, tl, 272, tl_n);       // P^T stored
+              tl_event(p, tl, 272, tl_n);       // tail P stored
             } else {
               mbar_wait(misc + MB_PV_DONE, (n_head + 2) & 1);
               tc_fence_after_sync();
             }
             if (t > 0) {
               if (t == 2) epi_o(tmem, sb, g, 1, (n_head + 1) & 1, inv_prev, q, part, lane);
-#if AFT_TC_TAILT == 2
-              else if (t == 3 && q < 2) epi_o_tail_sliced(tmem, sb, miscb, g, (n_head + 2) & 1, q, part, lane);
-#else
-              else if (t == 3 && q < kOtQuads) epi_o_tail(tmem, sb, g, (n_head + 2) & 1, q, part, lane);
-#endif
+              else if (t == 3 && q < 2) epi_o_tail(tmem, sb, miscb, g, (n_head + 2) & 1, q, part, lane);
               tc_fence_before_sync();
               fence_proxy_async_smem();
               warp_arrive(misc + MB_O_FREE + 8 * ((n_head + t - 1) & 1), lane);
@@ -1377,74 +996,12 @@ __global__ void __launch_bounds__(kTcThreads, 1) encoder_kernel(EncParams p) {
             }
           }
         }
-#else
-          float inv_prev = 0.f;
-#pragma unroll 1
-          for (int t = 0; t < 4; ++t) {
-            const bool active = t < 2 || tile2_active;
-            float sum = 0.f;
-            if (t < 3) {
-              mbar_wait(misc + MB_S_DONE, (n_head + t) & 1);
-              tc_fence_after_sync();
-              tl_event(p, tl, 230 + t, tl_n);   // S_DONE(t) seen
-              // The score row lives in registers from here to the P store.  It is defined and consumed inside ONE branch:
-              // a value defined under one `if (active)` and used under another would be loop-carried in the compiler's
-              // eyes and pin kSmCols registers for the whole kernel.
-              if (active) {
-                float v[kSmCols];
-                float m = softmax_load(tmem, q, part, v);
-                st_shared_f32(xmax_row + part * 512, m);
-                tc_fence_before_sync();
-                warp_arrive(misc + MB_S_LOADED, lane);
-                tl_event(p, tl, 240 + t, tl_n);   // S(t) loaded
-                named_bar_sync(1 + q, 32 * kParts);                          // exchange the partial row maxima
-#pragma unroll
-                for (int pp = 0; pp < kParts; ++pp) m = fmaxf(m, ld_shared_f32(xmax_row + pp * 512));
-                sum = softmax_exp(v, m);
-                tl_event(p, tl, 250 + t, tl_n);   // exponentials done
-                if (t > 0) { mbar_wait(misc + MB_PV_DONE, (n_head + t - 1) & 1); tc_fence_after_sync(); }   // P.V(t-1) has consumed P
-                tl_event(p, tl, 260 + t, tl_n);   // PV_DONE(t-1) seen
-                softmax_store(tmem, q, part, v);
-                st_shared_f32(xsum_row + part * 512, sum);
-              } else {
-                tc_fence_before_sync();
-                warp_arrive(misc + MB_S_LOADED, lane);
-                named_bar_sync(1 + q, 32 * kParts);
-                if (t > 0) { mbar_wait(misc + MB_PV_DONE, (n_head + t - 1) & 1); tc_fence_after_sync(); }
-              }
-              tc_fence_before_sync();
-              warp_arrive(misc + MB_P_READY, lane);
-              tl_event(p, tl, 270 + t, tl_n);   // P(t) stored
-            } else {
-              mbar_wait(misc + MB_PV_DONE, (n_head + 2) & 1);
-              tc_fence_after_sync();
-            }
-            if (t > 0) {
-              if (t - 1 < 2 || tile2_active) epi_o(tmem, sb, g, t - 1, (n_head + t - 1) & 1, inv_prev, q, part, lane);
-              tc_fence_before_sync();
-              fence_proxy_async_smem();
-              warp_arrive(misc + MB_O_FREE + 8 * ((n_head + t - 1) & 1), lane);
-            }
-            if (t < 3) {
-              named_bar_sync(1 + q, 32 * kParts);                          // exchange the partial row sums
-              float l_row = 0.f;
-#pragma unroll
-              for (int pp = 0; pp < kParts; ++pp) l_row += ld_shared_f32(xsum_row + pp * 512);
-              inv_prev = active ? rcp_approx(l_row) : 0.f;
-            }
-          }
-        }
-#endif
         // ---- out_proj epilogue: + bias + residual -> LayerNorm1 -> X
         tl_event(p, tl, 280, tl_n);   // waiting OUT_DONE
         mbar_wait(misc + MB_VEC_FULL, n_layer & 1);   // this layer's bias / LayerNorm vectors are in shared memory
 #pragma unroll 1
         for (int t = 0; t < 3; ++t) {   // per row tile: out_proj accumulators in -> LayerNorm1 rows out (FFN1 of the tile may start)
-          if (AFT_TC_SLICE2 && t == 2) {
-            mbar_wait(sb + OFF_BAR2 + MB2_OUT_DONE + 8 * t, n_layer & 1);
-            tc_fence_after_sync();
-            epi_ln_tail(tmem, sb, vec, 1, q, part, lane, miscb + MISC_XMAX);
-          } else if (t < 2 || tile2_active) {
+          if (t < 2 || tile2_active) {
             mbar_wait(sb + OFF_BAR2 + MB2_OUT_DONE + 8 * t, n_layer & 1);
             tc_fence_after_sync();
             epi_ln(tmem, sb, vec, 1, t, q, part, lane, t == 1 ? sb + OFF_LN1_XCHG : miscb + MISC_XMAX, nullptr, -1);
@@ -1463,14 +1020,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) encoder_kernel(EncParams p) {
           mbar_wait(misc + MB_F1_DONE, k & 1);
           tc_fence_after_sync();
           tl_event(p, tl, 300 + k, tl_n);   // F1_DONE(k) seen
-          if (AFT_TC_SLICE2 && t == 2) {   // third row tile, sliced: every quadrant holds 32 hidden units of the tail rows
-            f32x2 f[4];
-            act_tail_load(tmem, vec, pr, q, part, f);
-            tc_fence_before_sync();
-            warp_arrive(misc + MB_F1_FREE, lane);
-            if (pr == 1) mbar_wait(misc + MB_F2_DONE + 8 * t, 0);
-            act_tail_store(sb, p.activation, q, part, lane, f);
-          } else if (active) {   // accumulators defined and consumed inside one branch (see the softmax tiles)
+          if (active) {   // accumulators defined and consumed inside one branch (see the softmax tiles)
             f32x2 f[kActCols / 2];
             act_load(tmem, vec, pr, q, part, f);
             tc_fence_before_sync();
@@ -1490,11 +1040,7 @@ __global__ void __launch_bounds__(kTcThreads, 1) encoder_kernel(EncParams p) {
         tl_event(p, tl, 340, tl_n);   // LayerNorm2 start
 #pragma unroll 1
         for (int t = 0; t < 3; ++t) {   // per row tile: second completion of the tile's F2_DONE in this layer = final accumulators
-          if (AFT_TC_SLICE2 && t == 2) {
-            mbar_wait(misc + MB_F2_DONE + 8 * t, 1);
-            tc_fence_after_sync();
-            epi_ln_tail(tmem, sb, vec, 2, q, part, lane, miscb + MISC_XMAX);
-          } else if (t < 2 || tile2_active) {
+          if (t < 2 || tile2_active) {
             mbar_wait(misc + MB_F2_DONE + 8 * t, 1);
             tc_fence_after_sync();
             epi_ln(tmem, sb, vec, 2, t, q, part, lane, t == 1 ? sb + OFF_LN_XCHG : miscb + MISC_XMAX, nullptr, -1);
@@ -1668,18 +1214,6 @@ size_t tc_workspace_bytes(int64_t bc) {
          align_up_sz((size_t)bc * 3 * 2 * kS * sizeof(float), 1024);   // enhanced images | X images | adaptive features
 }
 
-// AFT_ENCODER=2|3 selects the encoder kernel (experiments / A-B runs); the default is compiled in
-#ifndef AFT_ENCODER_DEFAULT
-#define AFT_ENCODER_DEFAULT 2
-#endif
-static int encoder_version() {
-  static const int v = [] {
-    const char* e = getenv("AFT_ENCODER");
-    return e && (e[0] == '2' || e[0] == '3') ? e[0] - '0' : AFT_ENCODER_DEFAULT;
-  }();
-  return v;
-}
-
 bool tc_forward_chunk(const TcWeights& w, const FrontPack& front, const HeadPack& head, int activation, int sm_count,
                       const float2* pilots, const float* snr, const float* ds, const float* dop, const OutDst& out,
                       int64_t nsamples, void* workspace, cudaStream_t st, TcProfileHook hook) {
@@ -1704,13 +1238,9 @@ bool tc_forward_chunk(const TcWeights& w, const FrontPack& front, const HeadPack
   ep.timeline = g_timeline_arm;
   const unsigned grid = (unsigned)(nseq < sm_count ? nseq : sm_count);
   mark();
-  if (encoder_version() == 3) {
-    if (!tc_encoder3_launch(ximg, w.layers_dev, w.num_layers, activation, nseq, sm_count, st)) return false;
-  } else {
-    encoder_kernel<<<grid, kTcThreads, kTcSmemBytes, st>>>(ep);
-    count_launch();
-    if (!check_launch("encoder_kernel")) return false;
-  }
+  encoder_kernel<<<grid, kTcThreads, kTcSmemBytes, st>>>(ep);
+  count_launch();
+  if (!check_launch("encoder_kernel")) return false;
   mark();
   const bool ok = launch_head_tc(head, w.conv_head, ximg, enh, out, nsamples, sm_count, st);
   mark();
@@ -1835,10 +1365,9 @@ __global__ void __launch_bounds__(kTcThreads, 1) selftest_attn_kernel(const char
   if (warp == kMmaWarp) tmem_dealloc(tmem, 512);
 }
 
-// which = 3: the transposed tail tile (query rows 256..287) with the production helpers: S^T = K Q_tail^T, softmax over
-// the lanes, P^T -> Q image, O^T = V^T P^T, transposed store into the O image (head 0)
-// which = 4: the same tile with the sliced helpers (S slices per lane quadrant, P image in shared memory, M = 64 P.V)
-__global__ void __launch_bounds__(kTcThreads, 1) selftest_tail_kernel(const char* qkv_img, float* s_out, float* o_out, int sliced) {
+// which = 4: the tail tile (query rows 256..279) with the production helpers: S slices per lane quadrant, P image in
+// shared memory, M = 64 P.V, store into the O image (head 0)
+__global__ void __launch_bounds__(kTcThreads, 1) selftest_tail_kernel(const char* qkv_img, float* s_out, float* o_out) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const uint32_t sb = smem_u32(smem_raw);
   if ((sb & 1023u) != 0) __trap();
@@ -1864,11 +1393,11 @@ __global__ void __launch_bounds__(kTcThreads, 1) selftest_tail_kernel(const char
       bulk_g2s(sb + OFF_QKV, qkv_img, 3 * kQkvPart, misc + MB_X_FULL);
       mbar_wait(misc + MB_X_FULL, 0);
       tc_fence_after_sync();
-      if (sliced) issue_scores_tail_sliced(tmem, sb); else issue_scores_tail(tmem, sb);
+      issue_scores_tail(tmem, sb);
       mma_commit(misc + MB_S_DONE);
       mbar_wait(misc + MB_P_READY, 0);
       tc_fence_after_sync();
-      if (sliced) issue_pv_tail_sliced(tmem, sb, 1); else issue_pv_tail(tmem, sb, 1);
+      issue_pv_tail(tmem, sb, 1);
       mma_commit(misc + MB_PV_DONE);
     }
   } else {
@@ -1876,32 +1405,20 @@ __global__ void __launch_bounds__(kTcThreads, 1) selftest_tail_kernel(const char
     const int q = warp & 3, part = warp >> 2;
     mbar_wait(misc + MB_S_DONE, 0);
     tc_fence_after_sync();
-    if (sliced) {   // raw scores: thread (q, part, lane) holds query 256 + lane, 16 keys of its quadrant's slice at a time
-      const int nc = q == 0 ? 24 : 16, key0 = tail_key0(q) + part * nc;
-      for (int c0 = 0; c0 < nc; c0 += 8) {
-        uint32_t x[8];
-        tmem_ld_cols(tmem + ((uint32_t)(q * 32) << 16) + TM_S + key0 + c0, x);
-        tmem_wait_ld();
-        for (int j = 0; j < 8; ++j) s_out[(key0 + c0 + j) * 32 + lane] = __uint_as_float(x[j]);
-      }
-      softmax_tail_sliced(tmem, sb, miscb, misc + MB_S_LOADED, misc + MB_TAIL_MAX, 0, q, part, lane);
-    } else {
-      for (int b = 0; b < (q == 0 ? 3 : 2); ++b) {   // raw scores
-        uint32_t x[kTq];
-        tmem_ld_cols(tmem + ((uint32_t)(q * 32) << 16) + TM_S + b * 32 + part * kTq, x);
-        tmem_wait_ld();
-        const int key = b * 128 + q * 32 + lane;
-        if (key < kSPad)
-          for (int j = 0; j < kTq; ++j) s_out[key * 32 + part * kTq + j] = __uint_as_float(x[j]);
-      }
-      softmax_tail(tmem, sb, misc + MB_S_LOADED, q, part, lane);
+    // raw scores: thread (q, part, lane) holds query 256 + lane and 16 or 24 keys of its quadrant's slice, 8 at a time
+    const int nc = q == 0 ? 24 : 16, key0 = tail_key0(q) + part * nc;
+    for (int c0 = 0; c0 < nc; c0 += 8) {
+      uint32_t x[8];
+      tmem_ld_cols(tmem + ((uint32_t)(q * 32) << 16) + TM_S + key0 + c0, x);
+      tmem_wait_ld();
+      for (int j = 0; j < 8; ++j) s_out[(key0 + c0 + j) * 32 + lane] = __uint_as_float(x[j]);
     }
+    softmax_tail(tmem, sb, miscb, misc + MB_S_LOADED, misc + MB_TAIL_MAX, 0, q, part, lane);
     fence_proxy_async_smem();
     warp_arrive(misc + MB_P_READY, lane);
     mbar_wait(misc + MB_PV_DONE, 0);
     tc_fence_after_sync();
-    if (sliced) { if (q < 2) epi_o_tail_sliced(tmem, sb, miscb, 0, 1, q, part, lane); }
-    else if (q < kOtQuads) epi_o_tail(tmem, sb, 0, 1, q, part, lane);
+    if (q < 2) epi_o_tail(tmem, sb, miscb, 0, 1, q, part, lane);
     named_bar_sync(9, 32 * kComputeWarps);
     for (int i = threadIdx.x; i < 24 * 32; i += 32 * kComputeWarps) {
       const int r = 256 + i / 32, c = i % 32;
@@ -2089,7 +1606,7 @@ bool tc_selftest(int which, double* max_err, cudaStream_t st) {
     if (worst_s > 1e-3) { set_error("selftest attn tile %d: scores off by %g (outputs %g)", tile, worst_s, worst_o); }
     return true;
   }
-  if (which == 3 || which == 4) {
+  if (which == 4) {
     std::vector<float> Q(288 * 32), K(288 * 32), V(288 * 32);
     for (auto& v : Q) v = bf16_round_host(rng.next() * 1.5f);
     for (auto& v : K) v = bf16_round_host(rng.next() * 1.5f);
@@ -2114,7 +1631,7 @@ bool tc_selftest(int which, double* max_err, cudaStream_t st) {
     cudaMemsetAsync(dO, 0, 24 * 32 * sizeof(float), st);
     cudaMemcpyAsync(di, img.data(), 3 * kQkvPart, cudaMemcpyHostToDevice, st);
     cudaFuncSetAttribute(selftest_tail_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmemBytes);
-    selftest_tail_kernel<<<1, kTcThreads, kTcSmemBytes, st>>>(di, ds, dO, which == 4 ? 1 : 0);
+    selftest_tail_kernel<<<1, kTcThreads, kTcSmemBytes, st>>>(di, ds, dO);
     count_launch();
     std::vector<float> S(288 * 32), O(24 * 32);
     cudaMemcpyAsync(S.data(), ds, S.size() * sizeof(float), cudaMemcpyDeviceToHost, st);

@@ -40,12 +40,6 @@ bool tc_forward_chunk(const TcWeights& w, const FrontPack& front, const HeadPack
                       int64_t nsamples, void* workspace, cudaStream_t st, TcProfileHook hook);
 bool tc_selftest(int which, double* max_err, cudaStream_t st);
 
-// tc_encoder3.cu : encoder kernel v3 (three asynchronous row-tile streams per CTA, one thread per token row); same
-// operand images, same in-place contract on x_images as encoder_kernel.  Selected with AFT_ENCODER=3 (default: 2).
-bool tc_encoder3_launch(char* x_images, const TcLayer* layers_dev, int num_layers, int activation, int64_t nseq, int sm_count,
-                        cudaStream_t st);
-
-
 // tc_long.cu : the encoder for any sequence length (activations in global memory as per-row-tile operand images,
 // streaming attention).  h_in / h_out: fp32 [nseq * S][128] rows (may alias); workspace of tc_long_workspace_bytes().
 size_t tc_long_workspace_bytes(int64_t nseq, int S);

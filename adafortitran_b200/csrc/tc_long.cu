@@ -407,9 +407,7 @@ constexpr uint32_t ATM_S = 0, ATM_P = 64, ATM_O = 96;
 constexpr uint32_t kIdS = make_idesc_bf16(128, 64, false, false), kIdPV = make_idesc_bf16(128, 32, false, true);
 constexpr int kAtRegsCompute = 104, kAtRegsCtrl = 24;
 constexpr float kRescaleThreshold = 8.0f;
-#ifndef AFT_LONG_POLY
-#define AFT_LONG_POLY 4     // N > 0: one pair of exponentials in N runs on the FMA pipe (packed Cody-Waite + cubic, tc_math.cuh)
-#endif
+constexpr int kLongPoly = 4;   // one pair of exponentials in kLongPoly runs on the FMA pipe (packed Cody-Waite + cubic, tc_math.cuh)
 
 __global__ void __launch_bounds__(kAtThreads, 4) attn_long_kernel(AttnParams p) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -545,7 +543,7 @@ __global__ void __launch_bounds__(kAtThreads, 4) attn_long_kernel(AttnParams p) 
           const int c = i * 16 + 2 * jj;
           const f32x2 x2 = add2(pack2(v[c], v[c + 1]), negm2);
           f32x2 e2;
-          if (AFT_LONG_POLY > 0 && jj % (AFT_LONG_POLY > 0 ? AFT_LONG_POLY : 1) == (AFT_LONG_POLY > 0 ? AFT_LONG_POLY : 1) - 1) {
+          if (jj % kLongPoly == kLongPoly - 1) {
             e2 = ex2_poly2(x2);   // a share of the exponentials on the FMA pipe
           } else {
             float a, b;

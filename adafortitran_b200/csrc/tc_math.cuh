@@ -5,10 +5,6 @@
 #include "tc_layout.cuh"
 #include "tc_ptx.cuh"
 
-#ifndef AFT_TC_GELU_TANH
-#define AFT_TC_GELU_TANH 1  // 1: GELU through one MUFU.TANH (erf-fitted odd polynomial argument), 0: erf by Abramowitz-Stegun (2 MUFU)
-#endif
-
 namespace aft {
 namespace tcm {
 
@@ -35,20 +31,6 @@ __device__ __forceinline__ float rcp_approx(float x) {
   float y;
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
-}
-// GELU(x) = x Phi(x) with erf from Abramowitz-Stegun 7.1.26 (|err| <= 1.5e-7, far below the bf16 rounding of the
-// result): Phi(-|x|) = 0.5 poly(t) exp(-x^2/2), t = 1/(1 + p|x|/sqrt2);  gelu = max(x,0) - |x| Phi(-|x|).
-__device__ __forceinline__ float gelu_fast(float x) {
-  const float ax = fabsf(x);
-  const float t = rcp_approx(fmaf(ax, 0.3275911f * 0.70710678f, 1.0f));
-  const float e = ex2(x * x * (-0.5f * 1.4426950409f));
-  float p = 0.5f * 1.061405429f;
-  p = fmaf(p, t, 0.5f * -1.453152027f);
-  p = fmaf(p, t, 0.5f * 1.421413741f);
-  p = fmaf(p, t, 0.5f * -0.284496736f);
-  p = fmaf(p, t, 0.5f * 0.254829592f);
-  const float y = p * t * e;
-  return fmaf(-ax, y, fmaxf(x, 0.f));
 }
 // Packed fp32 pairs (FADD2 / FMUL2 / FFMA2 of sm_100): half the issue slots of the scalar forms, same rounding per lane.
 typedef unsigned long long f32x2;

@@ -115,27 +115,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   chaos_delay();
   if (!mbar_try_wait_for(bar, parity, AFT_TC_WAIT_HINT_NS)) mbar_wait_slow(bar, parity);
 }
-// Latency-critical waits (encoder v3: every hand-off between a stream's compute warps and its MMA issuer is on the stream's
-// critical path): poll with the plain try_wait -- the instruction itself blocks for a short, implementation-defined time --
-// instead of parking the warp in NANOSLEEP.SYNCS, whose wake-up costs several hundred cycles.  Same wall-clock budget.
-__device__ __forceinline__ void mbar_wait_spin(uint32_t bar, uint32_t parity) {
-  chaos_delay();
-#ifndef AFT_TC_SPIN_WAITS   // measured (encoder v3): polling costs more issue slots than the parked wait costs latency (60.9 vs 57.4 ms)
-  if (!mbar_try_wait_for(bar, parity, AFT_TC_WAIT_HINT_NS)) mbar_wait_slow(bar, parity);
-#else
-  for (int i = 0; i < 4096; ++i)
-    if (mbar_try_wait(bar, parity)) return;
-  mbar_wait_slow(bar, parity);
-#endif
-}
-// always polls (plain try_wait: the instruction itself blocks for a short, implementation-defined time); for the few warps
-// whose wake-up latency sits on every hand-off of a kernel (the MMA issuers of the encoder kernels)
-__device__ __forceinline__ void mbar_wait_poll(uint32_t bar, uint32_t parity) {
-  chaos_delay();
-  for (int i = 0; i < 8192; ++i)
-    if (mbar_try_wait(bar, parity)) return;
-  mbar_wait_slow(bar, parity);
-}
 // same contract; kept as a separate name for the roles whose waits are not latency critical (producer)
 __device__ __forceinline__ void mbar_wait_relaxed(uint32_t bar, uint32_t parity) {
   if (!mbar_try_wait_for(bar, parity, AFT_TC_WAIT_HINT_NS)) mbar_wait_slow(bar, parity);

@@ -33,7 +33,7 @@ def run(model, pilots, snr=None, ds=None, dop=None):
         return model(torch.from_numpy(pilots), md).cpu().numpy()
 
 
-@pytest.mark.parametrize("which,tol", [(0, 1e-4), (1, 5e-3), (2, 5e-3), (3, 2e-2), (4, 2e-2)])
+@pytest.mark.parametrize("which,tol", [(0, 1e-4), (1, 5e-3), (2, 5e-3), (4, 2e-2)])
 def test_tcgen05_building_blocks(which, tol):
     """UMMA GEMM tile (SWIZZLE_128B K-major descriptors, TMEM loads) and attention tiles (SWIZZLE_64B Q/K, MN-major V,
     P as TMEM A operand) against a double-precision host reference inside the library."""
@@ -252,29 +252,3 @@ def test_protocol_under_random_delays():
         res = json.loads(line[-1])
         assert r.returncode == 0, res
         assert res["lib"] == "libaft_b200_chaos.so" and res["wait_timeouts"] == 0 and res["rel_db_bf16_vs_fp32"] <= gate, res
-
-
-def test_encoder_v3_stream_kernel():
-    """The alternative encoder kernel (csrc/tc_encoder3.cu: three asynchronous row-tile streams, one thread per token row,
-    AFT_ENCODER=3) must give the product kernel's accuracy -- bf16 vs the fp32 path, which shares no code with either --
-    also under the chaos build (random delays before every mbarrier wait).  The selection is read once per process, hence
-    the subprocesses."""
-    import json, os, subprocess, sys
-    from adafortitran_b200.build import build as build_lib, lib_file
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    chaos = lib_file("chaos")
-    if not os.path.exists(chaos):
-        build_lib(variant="chaos")
-    for lib, batch, kind, gate in ((None, "160", "forti", -45.0), (None, "8", "ada", -36.0), (chaos, "296", "forti", -45.0)):
-        env = dict(os.environ, AFT_ENCODER="3")
-        if lib:
-            env["AFT_B200_LIB"] = lib
-        else:
-            env.pop("AFT_B200_LIB", None)
-        r = subprocess.run([sys.executable, os.path.join(root, "tools", "chaos_check.py"), batch, kind], env=env,
-                           capture_output=True, text=True, timeout=900)
-        line = [l for l in r.stdout.splitlines() if l.startswith("{")]
-        assert line, r.stdout + r.stderr
-        res = json.loads(line[-1])
-        assert r.returncode == 0, res
-        assert res["wait_timeouts"] == 0 and res["rel_db_bf16_vs_fp32"] <= gate, res

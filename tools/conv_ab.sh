@@ -2,7 +2,7 @@
 # GPU box: parity of the bf16 forward, conv-kernel timeline (tl build) and a short bench of both workloads.
 set -u
 mkdir -p gpurun_out
-unset AFT_ENCODER AFT_B200_LIB
+unset AFT_B200_LIB
 tag=${1:-conv}
 timeout 300 python tools/tc_check.py fwd 2>&1 | tail -4
 if [ -f adafortitran_b200/lib/libaft_b200_tl.so ]; then

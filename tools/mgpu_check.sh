@@ -3,7 +3,7 @@
 set -u
 N=${1:-2}
 mkdir -p gpurun_out
-unset AFT_ENCODER AFT_B200_LIB
+unset AFT_B200_LIB
 timeout 400 python -m torch.distributed.run --nnodes=1 --nproc-per-node $N --master-addr 127.0.0.1 --master-port 29512 bench.py --gpus $N --global-batch $((8192*N)) --steps 6 --warmup 3 --no-cpu-baseline > gpurun_out/mgpu_${N}.json 2> gpurun_out/mgpu_${N}.err
 python - <<PY
 import json

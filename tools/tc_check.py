@@ -9,7 +9,7 @@ from tests import util
 def selftests():
     torch.cuda.init(); torch.zeros(1, device="cuda")
     st = torch.cuda.current_stream().cuda_stream
-    for which in (0, 1, 2, 3, 4):
+    for which in (0, 1, 2, 4):
         err = C.c_double(-1)
         rc = _capi.lib().aft_selftest(which, C.byref(err), C.c_void_p(st))
         print(json.dumps({"selftest": which, "rc": rc, "max_err": err.value, "msg": _capi.lib().aft_last_error().decode()}), flush=True)
