@@ -45,7 +45,9 @@ Gates apply to each sample: fp32 <= 1e-5 normwise (ten times tighter than the pr
 output-relative error power <= -40 dB (FortiTran) / -34 dB (AdaFortiTran, random init: the raw metadata dominates the
 token features, DESIGN.md 5), against the oracle and against the fp32 path.  The bf16 gates cannot see a padding mask
 that is off by one key at S >= 65 (the extra key moves the output by -49 to -82 dB), nor a removed mask at S65 and
-S1025 (-47 / -46 dB); a removed mask is caught at S1, S129, S257, S258 and P64, an off-by-one mask at S1 and P64.  The Ada rows draw their metadata from the lower part of the reference's
+S1025 (-47 / -46 dB); a removed mask is caught at S1, S129, S257, S258 and P64, an off-by-one mask at S1 and P64.
+``tests/test_gpu_long_stages.py`` closes that gap: it checks each ``tc_long.cu`` kernel alone against fp64, with
+constructed weights under which the padding mask, the last key, the key ring and the rescale decide the result.  The Ada rows draw their metadata from the lower part of the reference's
 condition grid (SNR 0-30 dB, delay spread 50-200 ns, Doppler 200-600 Hz).
 """
 import time
